@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the B200 fusion-loss hot path (contract: see the task statement / DESIGN.md §6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[4], the configuration the headline metric is quoted on):
@@ -36,7 +36,14 @@ def parse():
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--no-extras', action='store_true', help='skip the e2e / metric-suite / cpu legs (profiling runs)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step returned to DIR/<name>.npy (see dump_outputs), to compare two builds')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs applies to --impl ours')
+    return args
 
 
 def measured_peak():
@@ -211,13 +218,14 @@ def main():
         l1 = fn1(a, b, y)                                # launches fusion_loss_ws_kernel<11,1,2>: loss values + d(total)/d imgf
         if ev:
             ev[1].record()
-        total = l1 + fn2(a, b, y, mode='max') + fn3(a, b, y, mode='max')      # the other two read the same launch
+        l2, l3 = fn2(a, b, y, mode='max'), fn3(a, b, y, mode='max')      # the other two read the same launch
+        total = l1 + l2 + l3
         total.backward()                                 # rescale_unit_kernel: in place, exits at once for unit upstream
         if ev:
             ev[2].record()
         if world > 1:                                    # the path's only collective: ONE 16-byte all-reduce, in place on the
             DU.reduce_loss_vector(ML.last_loss_vector(), world)      # kernel's own output vector (train.py:92-96 does four)
-        return y.grad
+        return y.grad, (l1, l2, l3, total)
 
     # ---- the same work straight through the C ABI: two-kernel path (forward, then recomputing backward) --------------
     cfg = ML._cfg(1.0, 'max', 'max', 'l1', 'l1', 1.0, 0.01, 0.1)
@@ -241,13 +249,16 @@ def main():
         torch.cuda.synchronize()
 
     def timed(run, steps):
-        """run(ev) records ev[0..2] around its two phases; returns (ms per step = max over ranks, mean ms of each phase)."""
+        """run(ev) records ev[0..2] around its two phases; returns (ms per step = max over ranks, mean ms of each phase,
+        what the last run returned)."""
         ev = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(steps)]
         t_begin, t_end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         sync_all()
         t_begin.record()
         for k in range(steps):
-            run(ev[k])
+            last = run(ev[k])
+            if k + 1 < steps:
+                del last            # freed before the next step allocates its gradient, as a discarded result would be
         t_end.record()
         sync_all()
         ms_total = t_begin.elapsed_time(t_end)
@@ -256,7 +267,7 @@ def main():
         tmax = torch.tensor([ms_total], device=dev)
         if world > 1:
             dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
-        return tmax.item() / steps, ms_a, ms_b
+        return tmax.item() / steps, ms_a, ms_b, last
 
     def two_kernel_step(ev):
         ev[0].record(); fwd(); ev[1].record(); bwd(); ev[2].record()
@@ -267,16 +278,19 @@ def main():
     sampler = ClockSampler(physical_gpu_index(local))
     sampler.start()
     c0 = L.launch_counts()
-    ms_step, ms_z, ms_rest = timed(step, args.steps)
+    ms_step, ms_z, ms_rest, last = timed(step, args.steps)
     c1 = L.launch_counts()
     clocks = sampler.stop()
     launches = {k: c1[k] - c0[k] for k in c1}
     assert launches['loss_single_pass'] == args.steps and launches['loss_fwd'] == 0 and launches['loss_bwd'] == 0, launches
-    grad_modules = step()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
+    del last
+    grad_modules = step()[0]
     vec = ML.last_loss_vector().double().cpu()
     for _ in range(3):
         fwd(); bwd()
-    ms_step2, ms_fwd, ms_bwd = timed(two_kernel_step, args.steps)
+    ms_step2, ms_fwd, ms_bwd, _ = timed(two_kernel_step, args.steps)
     total_mpix = GLOBAL_B * H * W / 1e6
     value = total_mpix / (ms_step * 1e-3)
 
@@ -360,6 +374,29 @@ def main():
         print(json.dumps(result))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_SAMPLE, DUMP_SEED, DUMP_CORNER = 1 << 22, 0, 512
+
+
+def dump_outputs(out_dir, grad, losses):
+    """What the last timed step handed its caller (rank 0's shard when N > 1), as float32 .npy files in `out_dir`:
+    loss.npy      [ssim, pixel, grad, total]: the three module outputs and their sum;
+    grad.npy      d(total)/d imgf at DUMP_SAMPLE flat indices drawn with numpy's default_rng(DUMP_SEED), sorted and
+                  de-duplicated (the whole gradient is 3.2 GB);
+    grad_corners.npy  the top-left DUMP_CORNER^2 block of the first image and the bottom-right one of the last, where the
+                  Sobel term's reflect padding and the SSIM window's valid region end.
+    The inputs come from a seeded generator, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    flat = grad.reshape(-1)
+    idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, flat.numel(), DUMP_SAMPLE))
+    c = DUMP_CORNER
+    arrays = {'loss': torch.stack([t.detach() for t in losses]),
+              'grad': flat[torch.from_numpy(idx).to(flat.device)],
+              'grad_corners': torch.stack([grad[0, 0, :c, :c], grad[-1, 0, -c:, -c:]])}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.float().cpu().numpy())
 
 
 def crop_parity_check(dev, ML, a, b, f):
