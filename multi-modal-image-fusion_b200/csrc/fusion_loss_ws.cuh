@@ -20,7 +20,7 @@
 //     port turned out to be the binding resource (a packed FFMA2 holds it for two cycles: issue 62 % + packed shadows 30 %
 //     = 92-94 % busy), so the hand-overs between groups are HARDWARE named barriers (bar.arrive / bar.sync: a blocked warp
 //     issues nothing) and only the TMA ring keeps mbarriers;
-//   * with the port saturated the only remaining lever is the instruction count per batch (2.73 k per 8 x 128 tile now).
+//   * with the port saturated the only remaining lever is the instruction count per batch (~2.6 k per 8 x 128 tile now).
 // Shared memory (213 KB of the SM's 227): 7-slot input ring (G3's combine reads rows three batches behind G0's prefetch),
 // double-buffered vbuf / cbuf / gbuf, one tbuf.
 #pragma once
@@ -39,9 +39,6 @@ constexpr unsigned kWsSleepNs = MMIF_WS_SLEEP_NS;
 #endif
 #ifndef MMIF_WS_H_UNROLL
 #define MMIF_WS_H_UNROLL 0
-#endif
-#ifndef MMIF_WS_V_ROLLED
-#define MMIF_WS_V_ROLLED 0
 #endif
 constexpr int kWsGroupBytes = 3 * kRB * kRPB * 4;
 
@@ -240,8 +237,39 @@ fusion_loss_ws_kernel(const __grid_constant__ CUtensorMap map1, const __grid_con
 
     if (grp == 0) {
         // =========================================================== G0: input ring (TMA producer), vertical moments
+        // Scatter form: each input row is loaded, shifted and multiplied ONCE and FMA'd into the WIN window rows it belongs
+        // to; the HALO window rows still open at the end of a batch are carried into the next one (a gather over the 18
+        // input rows of a batch would redo the loads and products of 10 of them).  Every window row still receives its
+        // taps in the order 0 .. WIN - 1, tap 0 as a multiply, so the sums are bit-identical to the gather form's.
+        static_assert(HALO <= 2 * kRB, "a batch's input rows must lie in three ring slots");
+        float2 acc[kRB + HALO][4];                      // window rows Rb .. Rb + 17 of batch b; [0, HALO) carried in
+        const float2 negc = f2(-sh.c.x, -sh.c.y);
+        // input row rr of the batch (ring row rp) -> tap rr - o of every open window row o <= rr
+        auto vrow = [&](const float* rp, const int rr) {
+            const float y = rp[2 * kWsRows * kRPB] - sh.cy;
+            float2 P[4];
+            P[0] = add2(f2(rp[0], rp[kWsRows * kRPB]), negc);
+            P[1] = mul2(P[0], P[0]);
+            P[2] = muls(y, P[0]);
+            P[3] = f2(y, y * y);
+            // window rows in ascending order (taps descending): then the last row of a batch finishes window row o before
+            // it writes row o + kRB, whose value is carried in the registers of row o, and the carry needs no moves
+#pragma unroll
+            for (int k = WIN - 1; k >= 0; --k) {
+                const int o = rr - k;
+                if (o >= 0) {
+#pragma unroll
+                    for (int m = 0; m < 4; ++m) acc[o][m] = (k == 0) ? muls(p.taps.w[0], P[m]) : fmas(p.taps.w[k], P[m], acc[o][m]);
+                }
+            }
+        };
         mbar_wait_wd(&sm.ring_full[0], 0);
         mbar_wait_wd(&sm.ring_full[1], 0);
+        {   // warm-up: input rows R0 .. R0 + HALO - 1 (ring slots 0 and 1) open window rows 0 .. HALO - 1 of batch 0
+            const float* q0 = &sm.ring[0][0][t + kVOFF];
+#pragma unroll
+            for (int rr = 0; rr < HALO; ++rr) vrow(q0 + rr * kRPB, rr);
+        }
 
         int slot = 0;                                   // b % kWsSlots
         for (int b = 0; b < nb; ++b) {
@@ -250,77 +278,23 @@ fusion_loss_ws_kernel(const __grid_constant__ CUtensorMap map1, const __grid_con
             // ---- V(b): vertical moments of window rows [Rb, Rb+8) -> vbuf[b & 1]
             if (b >= 2) nb_sync(NB_VEMPTY + (b & 1));             // H(b - 2) has read this vbuf
             {
-                // two passes of four output rows (14 input rows each) through one copy of the code: +10 rows of products
-                // per batch (~3 % of the FMA-pipe work) for half the instruction footprint and half the accumulators
+                // the batch's new input rows Rb + HALO .. Rb + HALO + 7 lie in the next two ring slots: two base pointers,
+                // constant row offsets, no per-row wrap arithmetic
                 float2* vb = sm.vbuf[b & 1];
-                const float2 negc = f2(-sh.c.x, -sh.c.y);
-                // the 18 input rows of the batch lie in three consecutive ring slots; a pass reads 14 of them as four
-                // segments of (up to) four rows whose base pointers are picked once per pass: no per-row wrap arithmetic
                 const int s1 = (slot + 1 == kWsSlots) ? 0 : slot + 1, s2 = (s1 + 1 == kWsSlots) ? 0 : s1 + 1;
-                const float* q0 = &sm.ring[0][slot * kRB][t + kVOFF];
-                const float* q2 = &sm.ring[0][s1 * kRB][t + kVOFF];
-                const float* q4 = &sm.ring[0][s2 * kRB][t + kVOFF];
-#if MMIF_WS_V_ROLLED
-                const float* q1 = q0 + 4 * kRPB;
-                const float* q3 = q2 + 4 * kRPB;
-#pragma unroll 1
-                for (int hv = 0; hv < 2; ++hv) {
-                    const float* sg[4] = {hv ? q1 : q0, hv ? q2 : q1, hv ? q3 : q2, hv ? q4 : q3};
-                    float2 acc[4][4];
+                const float* sg[3] = {nullptr, &sm.ring[0][s1 * kRB][t + kVOFF], &sm.ring[0][s2 * kRB][t + kVOFF]};
 #pragma unroll
-                    for (int rr = 0; rr < 4 + WIN - 1; ++rr) {
-                        const float* rp = sg[rr >> 2] + (rr & 3) * kRPB;
-                        const float y = rp[2 * kWsRows * kRPB] - sh.cy;
-                        float2 P[4];
-                        P[0] = add2(f2(rp[0], rp[kWsRows * kRPB]), negc);
-                        P[1] = mul2(P[0], P[0]);
-                        P[2] = muls(y, P[0]);
-                        P[3] = f2(y, y * y);
+                for (int rr = HALO; rr < kRB + HALO; ++rr) {
+                    vrow(sg[rr >> 3] + (rr & 7) * kRPB, rr);
+                    const int o = rr - HALO;                    // window row o has all its taps
 #pragma unroll
-                        for (int o = 0; o < 4; ++o) {
-                            const int k = rr - o;
-                            if (k >= 0 && k < WIN) {
-#pragma unroll
-                                for (int m = 0; m < 4; ++m) acc[o][m] = (k == 0) ? muls(p.taps.w[0], P[m]) : fmas(p.taps.w[k], P[m], acc[o][m]);
-                            }
-                        }
-                        if (rr >= WIN - 1) {
-                            const int o = rr - (WIN - 1);
-#pragma unroll
-                            for (int m = 0; m < 4; ++m) vb[o * kVPitch + m * kVCols + t] = acc[o][m];
-                        }
-                    }
-                    vb += 4 * kVPitch;
+                    for (int m = 0; m < 4; ++m) vb[o * kVPitch + m * kVCols + t] = acc[o][m];
                 }
-#else
-                {   // one pass of eight output rows over the 18 input rows (three ring slots, constant offsets inside a slot)
-                    const float* sg[3] = {q0, q2, q4};
-                    float2 acc[kRB][4];
 #pragma unroll
-                    for (int rr = 0; rr < kRB + WIN - 1; ++rr) {
-                        const float* rp = sg[rr >> 3] + (rr & 7) * kRPB;
-                        const float y = rp[2 * kWsRows * kRPB] - sh.cy;
-                        float2 P[4];
-                        P[0] = add2(f2(rp[0], rp[kWsRows * kRPB]), negc);
-                        P[1] = mul2(P[0], P[0]);
-                        P[2] = muls(y, P[0]);
-                        P[3] = f2(y, y * y);
+                for (int d = 0; d < HALO; ++d) {
 #pragma unroll
-                        for (int o = 0; o < kRB; ++o) {
-                            const int k = rr - o;
-                            if (k >= 0 && k < WIN) {
-#pragma unroll
-                                for (int m = 0; m < 4; ++m) acc[o][m] = (k == 0) ? muls(p.taps.w[0], P[m]) : fmas(p.taps.w[k], P[m], acc[o][m]);
-                            }
-                        }
-                        if (rr >= WIN - 1) {
-                            const int o = rr - (WIN - 1);
-#pragma unroll
-                            for (int m = 0; m < 4; ++m) vb[o * kVPitch + m * kVCols + t] = acc[o][m];
-                        }
-                    }
+                    for (int m = 0; m < 4; ++m) acc[d][m] = acc[d + kRB][m];
                 }
-#endif
             }
             nb_arrive(NB_VFULL + (b & 1));
             slot = (slot + 1 == kWsSlots) ? 0 : slot + 1;
