@@ -307,6 +307,21 @@ int mmif_widen_u8(const unsigned char* src, size_t n, float* dst, void* stream);
 /* dst[i] = float32(src[i]) / 255 in IEEE float32 division: the `uint8 / 255` scaling the reference's datasets apply on the host
  * (data/dataset.py via torchvision to_tensor) done on the device, bit-identical, so training sources can be shipped as bytes. */
 int mmif_widen_u8_unit(const unsigned char* src, size_t n, float* dst, void* stream);
+
+/* ---- bfloat16 / float16 images (an autocast training step: the network's output is bfloat16, or float16 with a
+ * GradScaler).  The loss kernels compute in float32; these two streaming entries sit around them.
+ * mmif_widen: dst[i] = float32(src[i]), exact (float16 subnormals, +-inf and NaN as torch.Tensor.float() gives them);
+ *   src: n elements of src_dtype (2-byte aligned), dst: n floats (4-byte aligned).
+ * mmif_narrow: dst[i] = round-to-nearest-even of scale[0] * src[i] to dst_dtype (scale: one DEVICE float, or NULL for
+ *   no multiply); the product is formed as the rescale of the single-pass backward forms it, so the result is that
+ *   backward's float32 gradient .to(dtype) bit for bit, overflow to +-inf in float16 included.  src and scale 4-byte,
+ *   dst 2-byte aligned.
+ * Both: MMIF_E_NULL for a null src / dst, MMIF_E_MODE for a dtype other than BF16 / F16, MMIF_E_ALIGN for a misaligned
+ * pointer; n == 0 launches nothing.  No synchronisation, no allocation.  Counted under MMIF_CNT_AUX. */
+enum { MMIF_DTYPE_F32 = 0, MMIF_DTYPE_BF16 = 1, MMIF_DTYPE_F16 = 2 };
+int mmif_widen(const void* src, int src_dtype, size_t n, float* dst, void* stream);
+int mmif_narrow(const float* src, const float* scale, size_t n, int dst_dtype, void* dst, void* stream);
+
 int mmif_eval_suite_u8(const unsigned char* a, const unsigned char* b, const unsigned char* f, int N, int H, int W,
                        double* out, float* dev_scratch, void* ws, size_t ws_bytes, void* stream);
 int mmif_eval_suite_u8_host(const unsigned char* a_host, const unsigned char* b_host, const unsigned char* f_host,

@@ -19,6 +19,7 @@ SYMBOLS = [
     'mmif_reflect_pad_bwd', 'mmif_metric_workspace_bytes', 'mmif_stats', 'mmif_hist', 'mmif_qabf', 'mmif_qabf_raw', 'mmif_ssim',
     'mmif_msssim', 'mmif_viff', 'mmif_eval_suite', 'mmif_eval_suite_host', 'mmif_ssim_maps', 'mmif_widen_u8', 'mmif_widen_u8_unit',
     'mmif_eval_suite_u8', 'mmif_eval_suite_u8_host', 'mmif_norm_workspace_bytes', 'mmif_norm_loss', 'mmif_norm_loss_bwd', 'mmif_test_post',
+    'mmif_widen', 'mmif_narrow',
 ]
 
 COMBINE = {'max': 0, 'avg': 1}
@@ -26,6 +27,7 @@ NORM = {'l1': 1, 'l2': 2}
 LOSS_HEAD, LOSS_PER_SAMPLE = 4, 6
 ST_COUNT, EN_COUNT, HIST_WORDS = 16, 12, 3 * 256 + 2 * 65536
 MSSSIM_DOUBLES, VIFF_DOUBLES, EVAL_METRICS = 22, 26, 16
+HALF_DTYPES = {torch.bfloat16: 1, torch.float16: 2}       # MMIF_DTYPE_BF16, MMIF_DTYPE_F16
 
 
 class MmifLossCfg(ctypes.Structure):
@@ -103,6 +105,8 @@ def load():
     lib.mmif_norm_workspace_bytes.argtypes = []
     lib.mmif_norm_loss.argtypes = [vp, sz, ci, cf, vp, vp, sz, vp]
     lib.mmif_norm_loss_bwd.argtypes = [vp, sz, ci, cf, vp, vp, vp]
+    lib.mmif_widen.argtypes = [vp, ci, sz, vp, vp]
+    lib.mmif_narrow.argtypes = [vp, vp, sz, ci, vp, vp]
     for name in SYMBOLS:
         getattr(lib, name)  # every declared symbol must be exported
     _lib = lib
@@ -211,6 +215,45 @@ def as_f32_3d(t, name='image'):
     """(N,1,H,W) / (N,H,W) / (H,W) float32 contiguous view -> (tensor, N, H, W)."""
     if t.dtype != torch.float32:
         raise MmifError(f'{name}: float32 expected, got {t.dtype}')
+    dims = _dims_3d(t, name)
+    return (t.contiguous(),) + dims
+
+
+def as_loss_f32(t, name='image'):
+    """Input of the loss modules -> float32 contiguous tensor: float32 as it is, bfloat16 / float16 (an autocast training
+    step) widened on the device by mmif_widen, which is exact.  Every other dtype raises."""
+    if t.dtype == torch.float32:
+        return t.contiguous()
+    code = HALF_DTYPES.get(t.dtype)
+    if code is None:
+        raise MmifError(f'{name}: float32, bfloat16 or float16 expected, got {t.dtype}')
+    require_cuda(t, name)
+    src = t.contiguous()
+    dst = torch.empty(src.shape, dtype=torch.float32, device=src.device)
+    call(src.device, load().mmif_widen, src.data_ptr(), code, src.numel(), dst.data_ptr(), stream_int(src.device))
+    return dst
+
+
+def as_loss_f32_3d(t, name='image'):
+    """as_f32_3d for the loss modules: bfloat16 / float16 images are accepted too and widened (as_loss_f32)."""
+    if t.dtype == torch.float32:
+        return as_f32_3d(t, name)
+    dims = _dims_3d(t, name)
+    return (as_loss_f32(t, name),) + dims
+
+
+def narrow_grad(g, dtype, scale=None):
+    """Gradient of a loss-module input: the float32 device tensor `g` itself for a float32 input, else
+    round-to-nearest-even of (scale[0] *) g to `dtype`, written by mmif_narrow.  scale: a float32 device scalar or None."""
+    if dtype == torch.float32 and scale is None:
+        return g
+    out = torch.empty(g.shape, dtype=dtype, device=g.device)
+    call(g.device, load().mmif_narrow, g.data_ptr(), scale.data_ptr() if scale is not None else None, g.numel(), HALF_DTYPES[dtype],
+         out.data_ptr(), stream_int(g.device))
+    return out
+
+
+def _dims_3d(t, name):
     if t.dim() == 4:
         if t.shape[1] != 1:
             raise MmifError(f'{name}: single-channel (N,1,H,W) expected, got {tuple(t.shape)}')
@@ -221,7 +264,7 @@ def as_f32_3d(t, name='image'):
         n, (h, w) = 1, t.shape
     else:
         raise MmifError(f'{name}: unsupported rank {t.dim()}')
-    return t.contiguous(), int(n), int(h), int(w)
+    return int(n), int(h), int(w)
 
 
 _REFERENCE_WINDOWS = [(11, 1.5), (17, 17 / 5), (9, 9 / 5), (5, 5 / 5), (3, 3 / 5)] + [(k, 1.5) for k in range(1, 11)] \

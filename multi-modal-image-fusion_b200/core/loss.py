@@ -16,8 +16,10 @@ operator + its adjoint, applied per pyramid level / per window for 'ms-ssim' / '
 windows 11/9/7/5/3 on the strip kernels and for ANY other window of 2..17 taps (odd or even) on the generic kernels
 (mmif_ssim_generic_*), with a dict that is differentiable w.r.t. both images through all three entries, per-sample or as
 size_average=False maps.  'msw-ssim' runs the same forward / backward kernels with the 11/9/7/5/3 windows and per-position
-weights.  Not built (raise NotImplementedError, never a silent fallback): gradients of the fused objective w.r.t. the
-sources, SSIM windows above 17 taps, MS_SSIM(size_average=False), MSW_SSIM(size_average=False) with windows other than 11/9/7/5/3.
+weights.  Every module takes float32, bfloat16 or float16 images (an autocast training step): a bfloat16 / float16 input is
+widened to float32 on the device on entry (exact, so the values are those of the float32 path on img.float()) and its
+gradient is narrowed from float32 to the input's dtype by mmif_narrow on exit.  Not built (raise NotImplementedError, never a
+silent fallback): gradients of the fused objective w.r.t. the sources, SSIM windows above 17 taps, MS_SSIM(size_average=False), MSW_SSIM(size_average=False) with windows other than 11/9/7/5/3.
 """
 import ctypes
 import threading
@@ -82,9 +84,9 @@ class _FusedObjective(torch.autograd.Function):
     @staticmethod
     def forward(ctx, img1, img2, imgf, cfg_key, want_grad):
         lib = L.load()
-        x1, B, H, W = L.as_f32_3d(img1, 'img1')
-        x2, _, _, _ = L.as_f32_3d(img2, 'img2')
-        y, _, _, _ = L.as_f32_3d(imgf, 'imgf')
+        x1, B, H, W = L.as_loss_f32_3d(img1, 'img1')
+        x2, _, _, _ = L.as_loss_f32_3d(img2, 'img2')
+        y, _, _, _ = L.as_loss_f32_3d(imgf, 'imgf')
         if x2.shape != x1.shape or y.shape != x1.shape:
             raise L.MmifError(f'shape mismatch: {tuple(img1.shape)} {tuple(img2.shape)} {tuple(imgf.shape)}')
         dev = y.device
@@ -100,7 +102,8 @@ class _FusedObjective(torch.autograd.Function):
         L.call(dev, fc.loss_fwd if fc is not None else lib.mmif_fusion_loss_fwd, x1.data_ptr(), x2.data_ptr(), y.data_ptr(), B, H, W,
                caddr if fc is not None else cref, out.data_ptr(), dF_unit.data_ptr() if want_grad else None, ws.data_ptr(),
                ws.numel(), stream)
-        ctx.save_for_backward(x1, x2, y)
+        # a bfloat16 / float16 input is kept as it came: only a recomputing backward needs its float32 widening again
+        ctx.save_for_backward(*(x if t.dtype == torch.float32 else t for t, x in ((img1, x1), (img2, x2), (imgf, y))))
         ctx.dF_unit = dF_unit
         ctx.single_pass = want_grad          # which kernel served the forward (the tests assert on it)
         ctx.cfg_key, ctx.dims, ctx.in_shape = cfg_key, (B, H, W), imgf.shape
@@ -114,9 +117,9 @@ class _FusedObjective(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_ssim, g_pix, g_grad, _g_ps):
         lib = L.load()
-        x1, x2, y = ctx.saved_tensors
+        s1, s2, sf = ctx.saved_tensors
         B, H, W = ctx.dims
-        dev = y.device
+        dev, dtype = sf.device, sf.dtype
         ups, ptrs = [], []
         for g in (g_ssim, g_pix, g_grad):       # device scalars as autograd hands them over: no stack / zeros launches
             if g is None:
@@ -128,7 +131,7 @@ class _FusedObjective(torch.autograd.Function):
             ups.append(g)
             ptrs.append(g.data_ptr())
         if not ups:
-            return None, None, torch.zeros(ctx.in_shape, dtype=torch.float32, device=dev), None, None
+            return None, None, torch.zeros(ctx.in_shape, dtype=dtype, device=dev), None, None
         _, cref, caddr = _cfg_ref(ctx.cfg_key, False)
         # The single-pass buffer is consumed by the first backward: it is rescaled IN PLACE (nothing to do at all for
         # the unit upstream of total.backward()) and handed to autograd; a second backward (retain_graph) recomputes.
@@ -136,6 +139,11 @@ class _FusedObjective(torch.autograd.Function):
         tok = getattr(ctx, 'memo_token', None)
         if tok is not None:
             tok[0] = False          # this graph has been backpropagated: a later call on the same tensors builds a fresh one
+        if dtype != torch.float32 and unit is not None and ptrs[0] is not None and ptrs[0] == ptrs[1] == ptrs[2]:
+            # total.backward() of a bfloat16 / float16 imgf (the same pointer test as mmif_fusion_loss_bwd3): the rescale of the
+            # single-pass buffer and the narrowing are one launch, the whole backward
+            return None, None, L.narrow_grad(unit, dtype, ups[0]).view(ctx.in_shape), None, None
+        x1, x2, y = (s if s.dtype == torch.float32 else L.as_loss_f32(s) for s in (s1, s2, sf))
         dF = unit if unit is not None else torch.empty_like(y)
         stream = L.stream_int(dev)
         ws = _loss_ws(lib, dev, stream, B, H, W)
@@ -143,7 +151,7 @@ class _FusedObjective(torch.autograd.Function):
         L.call(dev, fc.loss_bwd3 if fc is not None else lib.mmif_fusion_loss_bwd3, x1.data_ptr(), x2.data_ptr(), y.data_ptr(), B, H, W,
                caddr if fc is not None else cref, ptrs[0], ptrs[1], ptrs[2], unit.data_ptr() if unit is not None else None,
                dF.data_ptr(), ws.data_ptr(), ws.numel(), stream)
-        return None, None, dF.view(ctx.in_shape), None, None
+        return None, None, L.narrow_grad(dF, dtype).view(ctx.in_shape), None, None
 
 
 SINGLE_PASS = True   # set False to force the two-kernel (forward, then recomputing backward) path
@@ -161,7 +169,7 @@ class _Memo(threading.local):
     def lookup(self, img1, img2, imgf, cfg_key):
         want_grad = bool(SINGLE_PASS and imgf.requires_grad and torch.is_grad_enabled())    # the CALLER's grad mode
         key = (img1.data_ptr(), img1._version, img2.data_ptr(), img2._version, imgf.data_ptr(), imgf._version,
-               imgf.shape, imgf.device, cfg_key, imgf.requires_grad and torch.is_grad_enabled(), want_grad)
+               imgf.shape, imgf.device, imgf.dtype, cfg_key, imgf.requires_grad and torch.is_grad_enabled(), want_grad)
         # a hit needs the same tensors (identity + version) AND a graph that has not been backpropagated yet: the reference
         # builds a new graph on every call, so loss(...).backward() twice on the same tensors must keep working
         if self.key == key and self.token[0] and all(r() is t for r, t in zip(self.refs, (img1, img2, imgf))):
@@ -274,9 +282,9 @@ def _prep3(img1, img2, imgf):
         L.require_cuda(t, nm)
     if img1.requires_grad or img2.requires_grad:
         raise NotImplementedError('gradients w.r.t. the source images are not built (train.py never needs them)')
-    x1, B, H, W = L.as_f32_3d(img1.detach(), 'img1')
-    x2, _, _, _ = L.as_f32_3d(img2.detach(), 'img2')
-    y, _, _, _ = L.as_f32_3d(imgf.detach(), 'imgf')
+    x1, B, H, W = L.as_loss_f32_3d(img1.detach(), 'img1')
+    x2, _, _, _ = L.as_loss_f32_3d(img2.detach(), 'img2')
+    y, _, _, _ = L.as_loss_f32_3d(imgf.detach(), 'imgf')
     if x2.shape != x1.shape or y.shape != x1.shape:
         raise L.MmifError(f'shape mismatch: {tuple(img1.shape)} {tuple(img2.shape)} {tuple(imgf.shape)}')
     L.ensure_device(y.device)
@@ -293,7 +301,7 @@ class _WeightedSSIM(torch.autograd.Function):
         ps = _fwd_per_sample(x1, x2, y, data_range, win).to(torch.float32)
         gamma = ps[:, 2] / (ps[:, 2] + ps[:, 5]).clamp_(min=eps)
         ctx.save_for_backward(x1, x2, y, gamma)
-        ctx.data_range, ctx.in_shape, ctx.win = data_range, imgf.shape, win
+        ctx.data_range, ctx.in_shape, ctx.win, ctx.dtype = data_range, imgf.shape, win, imgf.dtype
         return (gamma * ps[:, 0]).mean() + ((1.0 - gamma) * ps[:, 3]).mean()
 
     @staticmethod
@@ -302,7 +310,7 @@ class _WeightedSSIM(torch.autograd.Function):
         pw = torch.stack([gamma, 1.0 - gamma], dim=1)
         g1 = g.to(torch.float32).reshape(1).contiguous()
         dF = _ssim_bwd_ex(x1, x2, y, ctx.data_range, g1, pw, 0, 1.0 / y.shape[0], ctx.win)
-        return None, None, dF.view(ctx.in_shape), None, None
+        return None, None, L.narrow_grad(dF, ctx.dtype).view(ctx.in_shape), None, None
 
 
 def _loss_sigma(win):
@@ -353,8 +361,8 @@ class _SSIMGeneric(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, img1, img2, data_range, win, size_average):
-        x, B, H, W = L.as_f32_3d(img1.detach(), 'img1')
-        y, _, _, _ = L.as_f32_3d(img2.detach(), 'img2')
+        x, B, H, W = L.as_loss_f32_3d(img1.detach(), 'img1')
+        y, _, _, _ = L.as_loss_f32_3d(img2.detach(), 'img2')
         if y.shape != x.shape:
             raise L.MmifError(f'shape mismatch: {tuple(img1.shape)} {tuple(img2.shape)}')
         L.ensure_device(x.device)
@@ -362,6 +370,7 @@ class _SSIMGeneric(torch.autograd.Function):
         k = min(int(win), H, W)                                    # loss.py:67-71
         ctx.save_for_backward(x, y)
         ctx.meta = (data_range, k, bool(size_average), img1.shape, img2.shape)
+        ctx.dtypes = (img1.dtype, img2.dtype)
         ctx.set_materialize_grads(False)
         if size_average:
             per = _generic_fwd(x, y, data_range, k).to(torch.float32)
@@ -376,7 +385,8 @@ class _SSIMGeneric(torch.autograd.Function):
             return None, None, None, None, None
         dx, dy = _generic_bwd(x, y, data_range, k, g_ssim, g_cs, g_sigma, not size_average, ctx.needs_input_grad[0],
                               ctx.needs_input_grad[1])
-        return (dx.view(s1) if dx is not None else None), (dy.view(s2) if dy is not None else None), None, None, None
+        return (L.narrow_grad(dx, ctx.dtypes[0]).view(s1) if dx is not None else None), \
+            (L.narrow_grad(dy, ctx.dtypes[1]).view(s2) if dy is not None else None), None, None, None
 
 
 class _PlainSSIM(torch.autograd.Function):
@@ -388,7 +398,7 @@ class _PlainSSIM(torch.autograd.Function):
         x1, x2, y = _prep3(img1, img2, imgf)
         ps = _fwd_per_sample(x1, x2, y, data_range).to(torch.float32)
         ctx.save_for_backward(x1, x2, y)
-        ctx.data_range, ctx.in_shape = data_range, imgf.shape
+        ctx.data_range, ctx.in_shape, ctx.dtype = data_range, imgf.shape, imgf.dtype
         return (ps[:, 0].mean() + ps[:, 3].mean()) * 0.5
 
     @staticmethod
@@ -397,7 +407,7 @@ class _PlainSSIM(torch.autograd.Function):
         g1 = g.to(torch.float32).reshape(1).contiguous()
         pw = torch.full((y.shape[0], 2), 0.5, dtype=torch.float32, device=y.device)
         dF = _ssim_bwd_ex(x1, x2, y, ctx.data_range, g1, pw, 0, 1.0 / y.shape[0])
-        return None, None, dF.view(ctx.in_shape), None
+        return None, None, L.narrow_grad(dF, ctx.dtype).view(ctx.in_shape), None
 
 
 class _SSIMDict(torch.autograd.Function):
@@ -408,8 +418,8 @@ class _SSIMDict(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, img1, img2, data_range, win=11):
-        x, B, H, W = L.as_f32_3d(img1.detach(), 'img1')
-        y, _, _, _ = L.as_f32_3d(img2.detach(), 'img2')
+        x, B, H, W = L.as_loss_f32_3d(img1.detach(), 'img1')
+        y, _, _, _ = L.as_loss_f32_3d(img2.detach(), 'img2')
         if y.shape != x.shape:
             raise L.MmifError(f'shape mismatch: {tuple(img1.shape)} {tuple(img2.shape)}')
         L.ensure_device(x.device)
@@ -417,6 +427,7 @@ class _SSIMDict(torch.autograd.Function):
         ps = _fwd_per_sample(x, x, y, data_range, win).to(torch.float32)
         ctx.save_for_backward(x, y)
         ctx.data_range, ctx.shape1, ctx.shape2, ctx.win = data_range, img1.shape, img2.shape, win
+        ctx.dtypes = (img1.dtype, img2.dtype)
         ctx.set_materialize_grads(False)
         return ps[:, 0].clone(), ps[:, 1].clone(), ps[:, 2].clone()
 
@@ -437,13 +448,13 @@ class _SSIMDict(torch.autograd.Function):
 
         g1 = g2 = None
         if ctx.needs_input_grad[1]:
-            g2 = wrt(x, y).view(ctx.shape2)
+            g2 = L.narrow_grad(wrt(x, y), ctx.dtypes[1]).view(ctx.shape2)
         if ctx.needs_input_grad[0]:
             g1 = wrt(y, x) if (g_ssim is not None or g_cs is not None) else None
             if g_sigma is not None:             # sigma = clamp(var(img1), 1e-4) depends on img1 only: the generic backward
                 ds, _ = _generic_bwd(x, y, ctx.data_range, ctx.win, None, None, g_sigma.reshape(-1), False, True, False)
                 g1 = ds if g1 is None else g1.add_(ds)
-            g1 = g1.view(ctx.shape1) if g1 is not None else None
+            g1 = L.narrow_grad(g1, ctx.dtypes[0]).view(ctx.shape1) if g1 is not None else None
         return g1, g2, None, None
 
 
@@ -508,6 +519,7 @@ class _MSSSIM(torch.autograd.Function):
         vc = v.clamp(min=eps)
         ms = torch.prod(vc ** wts.view(5, 1, 1), dim=0)              # (B, 2)
         ctx.levels, ctx.ranges, ctx.in_shape, ctx.use_padding, ctx.win = levels, ranges, imgf.shape, use_padding, win
+        ctx.dtype = imgf.dtype
         ctx.save_for_backward(v, vc, ms, wts)
         return ms[:, 0].contiguous(), ms[:, 1].contiguous()
 
@@ -528,7 +540,7 @@ class _MSSSIM(torch.autograd.Function):
             Bn, H, W = grads[lvl - 1].shape
             with torch.cuda.device(ms.device):
                 L.check(lib.mmif_halve_bwd(grads[lvl].data_ptr(), Bn, H, W, grads[lvl - 1].data_ptr(), L.stream_ptr(ms.device)))
-        return None, None, grads[0].view(ctx.in_shape), None, None, None
+        return None, None, L.narrow_grad(grads[0], ctx.dtype).view(ctx.in_shape), None, None, None
 
 
 class _MSWSSIM(torch.autograd.Function):
@@ -558,6 +570,7 @@ class _MSWSSIM(torch.autograd.Function):
             total = total + sums.view(B, 8)[:, 0].sum() / (B * (Hp - k + 1) * (Wp - k + 1))
         ctx.save_for_backward(x1, x2, y)
         ctx.data_range, ctx.win_sizes, ctx.in_shape, ctx.use_padding = data_range, tuple(win_sizes), imgf.shape, use_padding
+        ctx.dtype = imgf.dtype
         return (total / len(win_sizes)).to(torch.float32)
 
     @staticmethod
@@ -582,7 +595,25 @@ class _MSWSSIM(torch.autograd.Function):
             if p:
                 folded = _pad_bwd_raw(dst, p)
                 dF = folded if i == 0 else dF.add_(folded)
-        return None, None, dF.view(ctx.in_shape), None, None, None
+        return None, None, L.narrow_grad(dF, ctx.dtype).view(ctx.in_shape), None, None, None
+
+
+class _Widen(torch.autograd.Function):
+    """bfloat16 / float16 -> float32 whose backward narrows the float32 gradient once.  For a module that feeds one input to
+    several autograd nodes: their float32 gradients are summed in float32, as on the float32 path, before the narrowing."""
+
+    @staticmethod
+    def forward(ctx, x):
+        ctx.dtype = x.dtype
+        return L.as_loss_f32(x.detach(), 'img')
+
+    @staticmethod
+    def backward(ctx, g):
+        return L.narrow_grad(g.contiguous(), ctx.dtype)
+
+
+def _widen_shared(t):
+    return t if t.dtype == torch.float32 else _Widen.apply(t)
 
 
 class _ReflectPad(torch.autograd.Function):
@@ -592,11 +623,11 @@ class _ReflectPad(torch.autograd.Function):
     def forward(ctx, img, pad):
         lib = L.load()
         L.require_cuda(img, 'img')
-        x, B, H, W = L.as_f32_3d(img.detach(), 'img')
+        x, B, H, W = L.as_loss_f32_3d(img.detach(), 'img')
         out = torch.empty(B, 1, H + 2 * pad, W + 2 * pad, dtype=torch.float32, device=x.device)
         with torch.cuda.device(x.device):
             L.check(lib.mmif_reflect_pad(x.data_ptr(), B, H, W, pad, out.data_ptr(), L.stream_ptr(x.device)))
-        ctx.dims, ctx.pad, ctx.in_shape = (B, H, W), pad, img.shape
+        ctx.dims, ctx.pad, ctx.in_shape, ctx.dtype = (B, H, W), pad, img.shape, img.dtype
         return out
 
     @staticmethod
@@ -607,7 +638,7 @@ class _ReflectPad(torch.autograd.Function):
         out = torch.empty(B, H, W, dtype=torch.float32, device=g.device)
         with torch.cuda.device(g.device):
             L.check(lib.mmif_reflect_pad_bwd(g.data_ptr(), B, H, W, ctx.pad, out.data_ptr(), L.stream_ptr(g.device)))
-        return out.view(ctx.in_shape), None
+        return L.narrow_grad(out, ctx.dtype).view(ctx.in_shape), None
 
 
 def _pad3(img1, img2, imgf, win_size=11):
@@ -622,10 +653,10 @@ class _TV(torch.autograd.Function):
     def forward(ctx, x, norm, weight):
         lib = L.load()
         L.require_cuda(x, 'x')
-        if x.dim() < 2 or x.dtype != torch.float32:
-            raise L.MmifError('TVLoss needs a float32 tensor with at least 2 dims')
+        if x.dim() < 2 or (x.dtype != torch.float32 and x.dtype not in L.HALF_DTYPES):
+            raise L.MmifError('TVLoss needs a float32, bfloat16 or float16 tensor with at least 2 dims')
         h, w = x.shape[-2:]
-        xc = x.detach().contiguous().view(-1, h, w)
+        xc = L.as_loss_f32(x.detach(), 'x').view(-1, h, w)
         dev = x.device
         L.ensure_device(dev)
         out = torch.empty(1, dtype=torch.float64, device=dev)
@@ -635,7 +666,7 @@ class _TV(torch.autograd.Function):
             L.check(lib.mmif_tv_loss(xc.data_ptr(), n, h, w, L.NORM[norm], float(weight), out.data_ptr(), ws.data_ptr(), ws.numel(),
                                      L.stream_ptr(dev)))
         ctx.save_for_backward(xc)
-        ctx.norm, ctx.weight, ctx.in_shape = norm, weight, x.shape
+        ctx.norm, ctx.weight, ctx.in_shape, ctx.dtype = norm, weight, x.shape, x.dtype
         return out[0].to(torch.float32)
 
     @staticmethod
@@ -648,7 +679,7 @@ class _TV(torch.autograd.Function):
         with torch.cuda.device(xc.device):
             L.check(lib.mmif_tv_loss_bwd(xc.data_ptr(), n, h, w, L.NORM[ctx.norm], float(ctx.weight), g1.data_ptr(), gx.data_ptr(),
                                          L.stream_ptr(xc.device)))
-        return gx.view(ctx.in_shape), None, None
+        return L.narrow_grad(gx, ctx.dtype).view(ctx.in_shape), None, None
 
 
 def _check_norm(mode):
@@ -701,8 +732,8 @@ def ssim_maps(img1, img2, data_range):
     lib = L.load()
     for t, nm in ((img1, 'img1'), (img2, 'img2')):
         L.require_cuda(t, nm)
-    x, B, H, W = L.as_f32_3d(img1.detach(), 'img1')
-    y, _, _, _ = L.as_f32_3d(img2.detach(), 'img2')
+    x, B, H, W = L.as_loss_f32_3d(img1.detach(), 'img1')
+    y, _, _, _ = L.as_loss_f32_3d(img2.detach(), 'img2')
     if y.shape != x.shape:
         raise L.MmifError(f'shape mismatch: {tuple(img1.shape)} {tuple(img2.shape)}')
     dev = x.device
@@ -804,6 +835,7 @@ class MSW_SSIM(nn.Module):
             # window-MEAN clamped variances of the sources, one weighted SSIM per window size — 'w-ssim' with that window
             if any(not 2 <= int(k) <= 17 for k in self.win_sizes):
                 raise NotImplementedError('SSIM windows of 2..17 taps are built')
+            img1, img2, imgf = (_widen_shared(t) for t in (img1, img2, imgf))      # one input, one node per window
             acc = 0.0
             for k in self.win_sizes:
                 x1, x2, y = _pad3(img1, img2, imgf, int(k)) if self.use_padding else (img1, img2, imgf)
@@ -903,9 +935,7 @@ class _Norm(torch.autograd.Function):
     def forward(ctx, x, mode, weight):
         lib = L.load()
         L.require_cuda(x, 'x')
-        if x.dtype != torch.float32:
-            raise L.MmifError(f'NormLoss: float32 expected, got {x.dtype}')
-        xc = x.detach().contiguous()
+        xc = L.as_loss_f32(x.detach(), 'NormLoss')
         dev = xc.device
         L.ensure_device(dev)
         out = torch.empty(1, dtype=torch.float64, device=dev)
@@ -914,7 +944,7 @@ class _Norm(torch.autograd.Function):
             L.check(lib.mmif_norm_loss(xc.data_ptr(), xc.numel(), L.NORM[mode], float(weight), out.data_ptr(), ws.data_ptr(),
                                        ws.numel(), L.stream_ptr(dev)))
         ctx.save_for_backward(xc)
-        ctx.mode, ctx.weight, ctx.in_shape = mode, weight, x.shape
+        ctx.mode, ctx.weight, ctx.in_shape, ctx.dtype = mode, weight, x.shape, x.dtype
         return out[0].to(torch.float32)
 
     @staticmethod
@@ -926,7 +956,7 @@ class _Norm(torch.autograd.Function):
         with torch.cuda.device(xc.device):
             L.check(lib.mmif_norm_loss_bwd(xc.data_ptr(), xc.numel(), L.NORM[ctx.mode], float(ctx.weight), g1.data_ptr(),
                                            gx.data_ptr(), L.stream_ptr(xc.device)))
-        return gx.view(ctx.in_shape), None, None
+        return L.narrow_grad(gx, ctx.dtype).view(ctx.in_shape), None, None
 
 
 class NormLoss(nn.Module):

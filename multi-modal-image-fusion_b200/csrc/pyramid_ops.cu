@@ -1,6 +1,10 @@
 // Small data-movement operators around the stencil kernels: the MS-SSIM level step of the loss
 // (loss.py:147-153) and its adjoint, reflect padding (use_padding=True, loss.py:45-47) and its adjoint,
-// and the TVLoss backward (loss.py:347-358).
+// the TVLoss backward (loss.py:347-358), and the widening / narrowing between the float32 the loss kernels
+// compute in and the uint8 / bfloat16 / float16 images around them.
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include "common.cuh"
 
 namespace mmif {
@@ -80,32 +84,88 @@ __global__ void __launch_bounds__(256) tv_bwd_kernel(const float* __restrict__ x
     gx[((size_t)n * H + r) * W + c] = g * acc;
 }
 
-// ---- uint8 ingest (eval.py:182-194 decodes 8-bit images and widens them on the host; widening on the device
-// cuts the host->device traffic of an evaluation 4x).  16 pixels per thread: one 16-byte load, four 16-byte stores.
-// UNIT: divide by 255 in IEEE float32 division — bit-identical to the `uint8 -> float32 / 255` of the reference's input
-// pipeline (data/dataset.py through torchvision's to_tensor), so a training loop can ship 8-bit sources to the device.
-template <bool UNIT>
-__device__ __forceinline__ float widen1(unsigned v) { return UNIT ? __fdiv_rn((float)v, 255.0f) : (float)v; }
+// ---- Widening to float32, exact for every source type below.
+// uint8 ingest (eval.py:182-194 decodes 8-bit images and widens them on the host; widening on the device cuts the
+// host->device traffic of an evaluation 4x).  U8Unit divides by 255 in IEEE float32 division — bit-identical to the
+// `uint8 -> float32 / 255` of the reference's input pipeline (data/dataset.py through torchvision's to_tensor), so a
+// training loop can ship 8-bit sources to the device.
+// bfloat16 / float16 images of an autocast training step enter the float32 loss kernels the same way: the value is
+// what torch.Tensor.float() gives (float16 subnormals, +-inf and NaN included).
+// Each source type names its storage bits and the float32 value of one element's bits.
+struct SrcU8 {
+    using bits = unsigned char;
+    static __device__ __forceinline__ float widen1(unsigned v) { return (float)v; }
+};
+struct SrcU8Unit {
+    using bits = unsigned char;
+    static __device__ __forceinline__ float widen1(unsigned v) { return __fdiv_rn((float)v, 255.0f); }
+};
+struct SrcBF16 {
+    using bits = unsigned short;
+    static __device__ __forceinline__ float widen1(unsigned v) { return __uint_as_float(v << 16); }
+};
+struct SrcF16 {
+    using bits = unsigned short;
+    static __device__ __forceinline__ float widen1(unsigned v) { return __half2float(__ushort_as_half((unsigned short)v)); }
+};
 
-template <bool UNIT>
-__global__ void __launch_bounds__(256) widen_u8_kernel(const unsigned char* __restrict__ src, float* __restrict__ dst, size_t n, int vec) {
+// One 16-byte load per thread and iteration (16 uint8 or 8 half-width elements), float4 stores; vec = both pointers 16-byte
+// aligned, else element by element.
+template <typename S>
+__global__ void __launch_bounds__(256) widen_kernel(const typename S::bits* __restrict__ src, float* __restrict__ dst, size_t n, int vec) {
+    constexpr int kBits = 8 * (int)sizeof(typename S::bits), kPer = 128 / kBits;
+    constexpr unsigned kMask = (1u << kBits) - 1u;
     const size_t stride = (size_t)gridDim.x * blockDim.x;
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (vec) {
-        const size_t n16 = n >> 4;
+        const size_t nv = n / kPer;
         const uint4* s16 = reinterpret_cast<const uint4*>(src);
         float4* d4 = reinterpret_cast<float4*>(dst);
-        for (; i < n16; i += stride) {
+        for (; i < nv; i += stride) {
             const uint4 v = __ldg(s16 + i);
             const unsigned w[4] = {v.x, v.y, v.z, v.w};
+            float e[kPer];
 #pragma unroll
-            for (int k = 0; k < 4; ++k)
-                d4[4 * i + k] = make_float4(widen1<UNIT>(w[k] & 0xFF), widen1<UNIT>((w[k] >> 8) & 0xFF), widen1<UNIT>((w[k] >> 16) & 0xFF),
-                                            widen1<UNIT>(w[k] >> 24));
+            for (int k = 0; k < kPer; ++k) e[k] = S::widen1((w[k * kBits / 32] >> (k * kBits % 32)) & kMask);
+#pragma unroll
+            for (int k = 0; k < kPer / 4; ++k) d4[(kPer / 4) * i + k] = make_float4(e[4 * k], e[4 * k + 1], e[4 * k + 2], e[4 * k + 3]);
         }
-        for (size_t t = (n16 << 4) + (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) dst[t] = widen1<UNIT>(src[t]);
+        for (size_t t = nv * kPer + (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) dst[t] = S::widen1(src[t]);
     } else {
-        for (; i < n; i += stride) dst[i] = widen1<UNIT>(src[i]);
+        for (; i < n; i += stride) dst[i] = S::widen1(src[i]);
+    }
+}
+
+// ---- Narrowing of a float32 gradient to the bfloat16 / float16 of the image it belongs to: dst = RNE(scale[0] * src), the
+// product formed as rescale_unit_kernel forms it (g0 * v), so the result is that kernel's float32 gradient .to(dtype) bit
+// for bit, overflow to +-inf in float16 included (what a GradScaler detects).  scale == NULL: dst = RNE(src).
+template <typename D> __device__ __forceinline__ D narrow1(float v);
+template <> __device__ __forceinline__ __nv_bfloat16 narrow1<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ __half narrow1<__half>(float v) { return __float2half_rn(v); }
+
+// vec = src 16-byte and dst 8-byte aligned: one float4 load and one 8-byte store per thread and iteration.
+template <typename D>
+__global__ void __launch_bounds__(256) narrow_kernel(const float* __restrict__ src, const float* __restrict__ scale, D* __restrict__ dst,
+                                                     size_t n, int vec) {
+    const bool scaled = scale != nullptr;
+    const float g0 = scaled ? __ldg(scale) : 1.f;
+    auto one = [&](float v) { return narrow1<D>(scaled ? g0 * v : v); };
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (vec) {
+        const size_t n4 = n >> 2;
+        const float4* s4 = reinterpret_cast<const float4*>(src);
+        uint2* d4 = reinterpret_cast<uint2*>(dst);
+        for (; i < n4; i += stride) {
+            const float4 v = __ldcs(s4 + i);
+            const D o[4] = {one(v.x), one(v.y), one(v.z), one(v.w)};
+            uint2 u;
+            memcpy(&u, o, sizeof(u));
+            d4[i] = u;
+        }
+        for (size_t t = (n4 << 2) + (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) dst[t] = one(src[t]);
+    } else {
+        for (; i < n; i += stride) dst[i] = one(src[i]);
     }
 }
 
@@ -203,6 +263,20 @@ extern "C" int mmif_tv_loss_bwd(const float* x, int N, int H, int W, int norm, f
     return MMIF_OK;
 }
 
+// grid of the streaming kernels: one 16-byte source load per thread, at most 16 CTAs per SM (grid-stride beyond that)
+static unsigned stream_blocks(size_t n, size_t per_thread) {
+    const size_t blocks = (n / per_thread + 255) / 256;
+    return (unsigned)(blocks < 1 ? 1 : (blocks > 148 * 16 ? 148 * 16 : blocks));
+}
+template <typename S>
+static int widen_launch(const void* src, size_t n, float* dst, void* stream) {
+    const int vec = ((((uintptr_t)src) | ((uintptr_t)dst)) & 15) == 0;
+    widen_kernel<S><<<stream_blocks(n, 16 / sizeof(typename S::bits)), 256, 0, (cudaStream_t)stream>>>(
+        (const typename S::bits*)src, dst, n, vec);
+    mmif::count_launch(MMIF_CNT_AUX);
+    MMIF_CUDA(cudaGetLastError());
+    return MMIF_OK;
+}
 static int widen_impl(const unsigned char* src, size_t n, float* dst, void* stream, bool unit);
 extern "C" int mmif_widen_u8(const unsigned char* src, size_t n, float* dst, void* stream) { return widen_impl(src, n, dst, stream, false); }
 extern "C" int mmif_widen_u8_unit(const unsigned char* src, size_t n, float* dst, void* stream) { return widen_impl(src, n, dst, stream, true); }
@@ -210,11 +284,29 @@ static int widen_impl(const unsigned char* src, size_t n, float* dst, void* stre
     if (!src || !dst) { set_error("null pointer"); return MMIF_E_NULL; }
     if (((uintptr_t)dst) & 3) { set_error("dst must be 4-byte aligned"); return MMIF_E_ALIGN; }
     if (n == 0) return MMIF_OK;
-    const int vec = ((((uintptr_t)src) | ((uintptr_t)dst)) & 15) == 0;
-    size_t blocks = (n / 16 + 255) / 256;
-    blocks = blocks < 1 ? 1 : (blocks > 148 * 16 ? 148 * 16 : blocks);
-    if (unit) widen_u8_kernel<true><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(src, dst, n, vec);
-    else widen_u8_kernel<false><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(src, dst, n, vec);
+    return unit ? widen_launch<SrcU8Unit>(src, n, dst, stream) : widen_launch<SrcU8>(src, n, dst, stream);
+}
+extern "C" int mmif_widen(const void* src, int src_dtype, size_t n, float* dst, void* stream) {
+    if (!src || !dst) { set_error("null pointer"); return MMIF_E_NULL; }
+    if (src_dtype != MMIF_DTYPE_BF16 && src_dtype != MMIF_DTYPE_F16) { set_error("widen: source dtype %d is not BF16 / F16", src_dtype); return MMIF_E_MODE; }
+    if ((((uintptr_t)src) & 1) || (((uintptr_t)dst) & 3)) { set_error("widen: src must be 2-byte, dst 4-byte aligned"); return MMIF_E_ALIGN; }
+    if (n == 0) return MMIF_OK;
+    return src_dtype == MMIF_DTYPE_BF16 ? widen_launch<SrcBF16>(src, n, dst, stream) : widen_launch<SrcF16>(src, n, dst, stream);
+}
+extern "C" int mmif_narrow(const float* src, const float* scale, size_t n, int dst_dtype, void* dst, void* stream) {
+    if (!src || !dst) { set_error("null pointer"); return MMIF_E_NULL; }
+    if (dst_dtype != MMIF_DTYPE_BF16 && dst_dtype != MMIF_DTYPE_F16) { set_error("narrow: destination dtype %d is not BF16 / F16", dst_dtype); return MMIF_E_MODE; }
+    if (((((uintptr_t)src) | ((uintptr_t)scale)) & 3) || (((uintptr_t)dst) & 1)) {
+        set_error("narrow: src and scale must be 4-byte, dst 2-byte aligned");
+        return MMIF_E_ALIGN;
+    }
+    if (n == 0) return MMIF_OK;
+    const int vec = (((uintptr_t)src) & 15) == 0 && (((uintptr_t)dst) & 7) == 0;
+    const unsigned blocks = stream_blocks(n, 4);
+    if (dst_dtype == MMIF_DTYPE_BF16)
+        narrow_kernel<__nv_bfloat16><<<blocks, 256, 0, (cudaStream_t)stream>>>(src, scale, (__nv_bfloat16*)dst, n, vec);
+    else
+        narrow_kernel<__half><<<blocks, 256, 0, (cudaStream_t)stream>>>(src, scale, (__half*)dst, n, vec);
     mmif::count_launch(MMIF_CNT_AUX);
     MMIF_CUDA(cudaGetLastError());
     return MMIF_OK;
