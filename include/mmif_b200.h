@@ -240,6 +240,17 @@ enum { /* mmif_stats output, per pair */
 };
 int mmif_stats(const float* a, const float* b, const float* f, int N, int H, int W, double* out,
                void* ws, size_t ws_bytes, void* stream);
+/* Gradient of sum_c gout[c] * stat[c] over the MMIF_ST_* columns of the batch row `row` (device, MMIF_ST_COUNT
+ * doubles: what mmif_stats returns for N = 1, the whole-batch combination for N > 1).  gout: device, MMIF_ST_COUNT
+ * floats.  da / db / df: device, N*H*W floats each, any of them NULL (not computed, not written).
+ * The batch is one population (global means, variances, covariances); the AG / SF forward differences stay inside a
+ * sample.  Where the reference's autograd gives NaN so does this: a zero sd or a 0/0 correlation puts NaN on every pixel
+ * of the images it involves, an AG stencil with equal pixels on its three pixels.  A column whose gout is exactly 0
+ * contributes nothing.  Checks of mmif_stats plus MMIF_E_NULL for a null row / gout and MMIF_E_ALIGN for a row that is
+ * not 8-byte or a gout / gradient that is not 4-byte aligned; all three outputs NULL launches nothing.  No allocation,
+ * no synchronisation; one launch, counted under MMIF_CNT_METRIC. */
+int mmif_stats_bwd(const float* a, const float* b, const float* f, int N, int H, int W, const double* row,
+                   const float* gout, float* da, float* db, float* df, void* stream);
 
 enum { /* mmif_hist entropy outputs, per pair */
     MMIF_EN_A = 0, MMIF_EN_B = 1, MMIF_EN_F = 2, /* calc_entropy      metric.py:119-125 (float32 arithmetic) */

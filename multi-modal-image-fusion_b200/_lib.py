@@ -19,7 +19,7 @@ SYMBOLS = [
     'mmif_reflect_pad_bwd', 'mmif_metric_workspace_bytes', 'mmif_stats', 'mmif_hist', 'mmif_qabf', 'mmif_qabf_raw', 'mmif_ssim',
     'mmif_msssim', 'mmif_viff', 'mmif_eval_suite', 'mmif_eval_suite_host', 'mmif_ssim_maps', 'mmif_widen_u8', 'mmif_widen_u8_unit',
     'mmif_eval_suite_u8', 'mmif_eval_suite_u8_host', 'mmif_norm_workspace_bytes', 'mmif_norm_loss', 'mmif_norm_loss_bwd', 'mmif_test_post',
-    'mmif_widen', 'mmif_narrow',
+    'mmif_widen', 'mmif_narrow', 'mmif_stats_bwd',
 ]
 
 COMBINE = {'max': 0, 'avg': 1}
@@ -87,6 +87,7 @@ def load():
     lib.mmif_metric_workspace_bytes.restype = sz
     lib.mmif_metric_workspace_bytes.argtypes = [ci, ci, ci]
     lib.mmif_stats.argtypes = [vp, vp, vp, ci, ci, ci, vp, vp, sz, vp]
+    lib.mmif_stats_bwd.argtypes = [vp, vp, vp, ci, ci, ci, vp, vp, vp, vp, vp, vp]
     lib.mmif_hist.argtypes = [vp, vp, vp, ci, ci, ci, vp, vp, vp, sz, vp]
     lib.mmif_qabf.argtypes = [vp, vp, vp, ci, ci, ci, cf, vp, vp, sz, vp]
     lib.mmif_qabf_raw.argtypes = [vp, vp, vp, ci, ci, ci, cf, vp, vp, sz, vp]

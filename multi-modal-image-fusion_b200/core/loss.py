@@ -317,12 +317,13 @@ def _loss_sigma(win):
     return 1.5 if win == 11 else 0.15 * (win - 1)        # loss.py:34
 
 
-def _generic_fwd(x, y, data_range, win, want_maps=False):
-    """mmif_ssim_generic_fwd on (B,H,W) device tensors -> (B,3) float64 per-sample [ssim, cs, sigma], or the three maps."""
+def _generic_fwd(x, y, data_range, win, want_maps=False, sigma=None):
+    """mmif_ssim_generic_fwd on (B,H,W) device tensors -> (B,3) float64 per-sample [ssim, cs, sigma], or the three maps.
+    sigma: the window's Gaussian sigma, by default the loss rule (the metric functions pass 1.5)."""
     lib = L.load()
     B, H, W = y.shape
     dev = y.device
-    sigma = _loss_sigma(win)
+    sigma = _loss_sigma(win) if sigma is None else sigma
     L.ensure_window_taps(win, sigma)
     if want_maps:
         maps = [torch.empty(B, 1, H - win + 1, W - win + 1, dtype=torch.float32, device=dev) for _ in range(3)]
@@ -336,12 +337,13 @@ def _generic_fwd(x, y, data_range, win, want_maps=False):
     return per
 
 
-def _generic_bwd(x, y, data_range, win, g_ssim, g_cs, g_sigma, maps, want_dx, want_dy):
-    """mmif_ssim_generic_bwd: upstream gradients (per-sample (B,) or per-position maps, any may be None) -> (dx, dy)."""
+def _generic_bwd(x, y, data_range, win, g_ssim, g_cs, g_sigma, maps, want_dx, want_dy, sigma=None):
+    """mmif_ssim_generic_bwd: upstream gradients (per-sample (B,) or per-position maps, any may be None) -> (dx, dy).
+    sigma: the window's Gaussian sigma, by default the loss rule (the metric functions pass 1.5)."""
     lib = L.load()
     B, H, W = y.shape
     dev = y.device
-    sigma = _loss_sigma(win)
+    sigma = _loss_sigma(win) if sigma is None else sigma
     L.ensure_window_taps(win, sigma)
     gs = [None if g is None else g.to(device=dev, dtype=torch.float32).contiguous() for g in (g_ssim, g_cs, g_sigma)]
     coef = torch.empty(lib.mmif_ssim_generic_coef_doubles(B, H, W, int(win)), dtype=torch.float64, device=dev)

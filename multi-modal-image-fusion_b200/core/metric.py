@@ -9,6 +9,15 @@ by tensor identity) and ALL arithmetic runs on the GPU — there is no CPU compu
 ``eval_metrics_batch`` is the batched entry (N pairs per launch) the sharded evaluation and the
 benchmark use; the per-function drop-ins share kernel results through a small per-pair memo so
 the 20-odd calls of ``eval_metrics`` (eval.py:29-75) cost one launch per kernel family.
+
+Gradients, as the reference's torch ops give them: with grad mode on and an argument that requires grad,
+``calc_mean / std / ag / sf / mse / cc / scd`` (``mmif_stats_bwd``, one launch per call's backward),
+``calc_psnr`` (torch arithmetic on the mse tensor), ``calc_ssim`` (means, ``full=True`` and the 11-tap maps) and
+``calc_msssim`` (the SSIM backward kernels per level, plus the padding and pooling adjoints) are differentiable
+w.r.t. every image argument.  A batch is one population, as for the values.  The forward is the no-grad call
+itself (same memo entry, same launches, equal values); the gradient reaches exactly the tensors passed to the call,
+on their device (CPU inputs get CPU float32 gradients).  Qabf / Nabf / Labf, VIFF and the histogram family stay
+detached; the batched entries below take no gradient.
 """
 import ctypes
 import math
@@ -49,7 +58,7 @@ class _UploadCache:
         for ref, ver, dev in self.items:
             if ref() is t and ver == t._version:
                 return dev
-        dev = _staged_upload(t, _default_device())
+        dev = _staged_upload(t.detach(), _default_device())
         self.items.append((weakref.ref(t), t._version, dev))
         if len(self.items) > self.cap:
             self.items.pop(0)
@@ -214,9 +223,9 @@ def _combine_batch(kind, val, part, extra):
     raise L.MmifError(f'no batch rule for {kind}')
 
 
-def _rows(ent, home, part=None):
-    """The float64 row(s) of a memo entry where the caller lives: the device tensor, or its single host copy.  A batch
-    (N > 1) is first combined into the ONE row the reference's function returns for it (`_combine_batch`)."""
+def _dev_rows(ent, part=None):
+    """The float64 device row(s) of a memo entry; a batch (N > 1) is first combined into the ONE row the reference's
+    function returns for it (`_combine_batch`)."""
     val = ent[2] if part is None else ent[2][part]
     n = (ent[2][1] if ent[0][0] == 'hist' else val).shape[0]
     if ent[3] is None:
@@ -225,6 +234,13 @@ def _rows(ent, home, part=None):
         if ('g', part) not in ent[3]:
             ent[3][('g', part)] = _combine_batch(ent[0][0], ent[2], part, math.prod(ent[0][-1][2]))
         val = ent[3][('g', part)]
+    return val
+
+
+def _rows(ent, home, part=None):
+    """The float64 row(s) of a memo entry where the caller lives: the device tensor (`_dev_rows`), or its single host
+    copy."""
+    val = _dev_rows(ent, part)
     if home.type != 'cpu':
         return val if val.device == home else val.to(home)
     if ('h', part) not in ent[3]:
@@ -438,6 +454,235 @@ def _viff3(a, b, f):
     return _memo.get('viff', (a, b, f), None, run)
 
 
+# ---- gradients (reference semantics: core/metric.py's torch ops under autograd) ----
+def _grad_wanted(*args):
+    """A graph node is built only with grad mode on and an argument that requires grad; otherwise the call path and its
+    launches are the no-grad ones."""
+    return torch.is_grad_enabled() and any(t.requires_grad for t in args)
+
+
+def _dev_imgs(tr):
+    """Detached float32 (N,H,W) device images of a triple (CPU tensors: the upload cache's copies) + (N,H,W)."""
+    imgs, shape, _ = _prep(*tr)
+    return [t.detach().view(shape) for t in imgs], shape
+
+
+# statistics column -> the triple slots (0: a, 1: b, 2: f) it depends on
+_ST_DEPS = {0: (2,), 1: (2,), 2: (2,), 3: (2,), 4: (0, 2), 5: (1, 2), 6: (0, 2), 7: (1, 2), 8: (0, 1, 2)}
+
+
+class _StatFn(torch.autograd.Function):
+    """Column `col` of the statistics row of the triple `tr` (the no-grad value, from the same memo entry), differentiable
+    w.r.t. the call's arguments `args`, args[k] being the triple slot slots[k].  Backward: one mmif_stats_bwd launch with
+    a one-hot upstream gradient, on the device row."""
+
+    @staticmethod
+    def forward(ctx, tr, col, slots, *args):
+        ent = _stats(*tr)
+        out = _scalar(_rows(ent, args[0].device), col)
+        imgs, shape = _dev_imgs(tr)
+        ctx.save_for_backward(_dev_rows(ent), *imgs)
+        ctx.col, ctx.slots, ctx.shape = col, slots, shape
+        ctx.args = [(t.shape, t.device) for t in args]
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        row, a, b, f = ctx.saved_tensors
+        dev = a.device
+        gout = torch.zeros(L.ST_COUNT, dtype=torch.float32, device=dev)
+        gout[ctx.col] = g.to(device=dev, dtype=torch.float32)
+        outs = [None, None, None]
+        for k, s in enumerate(ctx.slots):
+            if ctx.needs_input_grad[3 + k] and s in _ST_DEPS[ctx.col] and outs[s] is None:
+                outs[s] = torch.empty(ctx.shape, dtype=torch.float32, device=dev)
+        if any(o is not None for o in outs):
+            n, h, w = ctx.shape
+            L.call(dev, L.load().mmif_stats_bwd, a.data_ptr(), b.data_ptr(), f.data_ptr(), n, h, w, row.data_ptr(),
+                   gout.data_ptr(), *(o.data_ptr() if o is not None else None for o in outs), L.stream_int(dev))
+        grads = []
+        for k, s in enumerate(ctx.slots):
+            shape, device = ctx.args[k]
+            if not ctx.needs_input_grad[3 + k]:
+                grads.append(None)
+            elif outs[s] is None:             # a slot this column does not depend on
+                grads.append(torch.zeros(shape, dtype=torch.float32, device=device))
+            else:
+                d = outs[s].view(shape)
+                grads.append(d if d.device == device else d.to(device))
+        return (None, None, None) + tuple(grads)
+
+
+def _stat(tr, col, slots, *args):
+    """Column `col` of the statistics of triple `tr` for a call on `args` (args[k] = tr[slots[k]])."""
+    if _grad_wanted(*args):
+        return _StatFn.apply(tr, col, slots, *args)
+    return _scalar(_rows(_stats(*tr), args[0].device), col)
+
+
+_MS_WEIGHTS = (0.0448, 0.2856, 0.3001, 0.2363, 0.1333)       # metric.py:372
+
+
+def _ssim_mean_grads(x, y, k, data_range, g_ssim, g_cs, want_x, want_y, strip=True):
+    """d/dx, d/dy of g_ssim * mean(ssim map) + g_cs * mean(cs map) over the whole (N,H,W) batch (metric.py:316-364) with a
+    k-tap window of sigma 1.5; g_*: float32 device scalars or None.  11 taps (and `strip`): the strip kernels, once per
+    wanted image (SSIM and CS are symmetric: the gradient w.r.t. either image is the fused-image gradient with the other as
+    the source); any shrunk window, or strip=False: the generic kernels (double arithmetic) with sigma 1.5 (the strip
+    kernels' 9/7/5/3-tap windows follow the loss rule)."""
+    from . import loss as ML
+    n = x.shape[0]
+    if k == 11 and strip:
+        pw = torch.zeros(n, 2, dtype=torch.float32, device=x.device)
+        pw[:, 0] = 1.0
+
+        def wrt(src, tgt):
+            out = None
+            for g, cs_only in ((g_ssim, 0), (g_cs, 1)):
+                if g is not None:
+                    d = ML._ssim_bwd_ex(src, src, tgt, data_range, g.reshape(1).contiguous(), pw, cs_only, 1.0 / n, 11)
+                    out = d if out is None else out.add_(d)
+            return out
+        return (wrt(y, x) if want_x else None), (wrt(x, y) if want_y else None)
+    L.ensure_window_taps(k, 1.5)
+    per = [None if g is None else (g.reshape(1) / n).expand(n) for g in (g_ssim, g_cs)]
+    return ML._generic_bwd(x, y, data_range, k, per[0], per[1], None, False, want_x, want_y, sigma=1.5)
+
+
+def _ssim_level_grads(x, y, win, data_range, use_padding, g_ssim, g_cs, want_x, want_y, strip=True):
+    """_ssim_mean_grads of one calc_ssim level: window min(win, H, W) (metric.py:323-325), use_padding reflect-pads by
+    half of it first (metric.py:305-311) and folds the gradients back."""
+    from . import loss as ML
+    h, w = x.shape[-2:]
+    k = min(int(win), h, w)
+    p = k // 2 if use_padding else 0
+    if p:
+        x, y = _pad_dev(x, p), _pad_dev(y, p)
+    dx, dy = _ssim_mean_grads(x, y, k, data_range, g_ssim, g_cs, want_x, want_y, strip)
+    if p:
+        dx = ML._pad_bwd_raw(dx, p) if dx is not None else None
+        dy = ML._pad_bwd_raw(dy, p) if dy is not None else None
+    return dx, dy
+
+
+def _as_dev_scalar(g, dev):
+    return None if g is None else g.to(device=dev, dtype=torch.float32)
+
+
+class _SSIMFn(torch.autograd.Function):
+    """calc_ssim(x, y, size_average=True): (ssim, cs) of the pair (tr[slot], tr[2]) from the memo entry, differentiable
+    w.r.t. x and y."""
+
+    @staticmethod
+    def forward(ctx, tr, slot, win, data_range, use_padding, x, y):
+        r = _rows(_ssim2(*tr, win, data_range, use_padding), x.device)
+        imgs, _ = _dev_imgs(tr)
+        ctx.save_for_backward(imgs[slot], imgs[2])
+        ctx.cfg, ctx.args = (win, data_range, use_padding), [(t.shape, t.device) for t in (x, y)]
+        ctx.set_materialize_grads(False)
+        return _scalar(r, 2 * slot), _scalar(r, 2 * slot + 1)
+
+    @staticmethod
+    def backward(ctx, g_ssim, g_cs):
+        x, y = ctx.saved_tensors
+        if g_ssim is None and g_cs is None:
+            return (None,) * 7
+        win, data_range, use_padding = ctx.cfg
+        dx, dy = _ssim_level_grads(x, y, win, data_range, use_padding, _as_dev_scalar(g_ssim, x.device),
+                                   _as_dev_scalar(g_cs, x.device), ctx.needs_input_grad[5], ctx.needs_input_grad[6])
+        return (None,) * 5 + tuple(None if d is None else d.view(s).to(dv) for d, (s, dv) in zip((dx, dy), ctx.args))
+
+
+class _SSIMMapFn(torch.autograd.Function):
+    """calc_ssim(x, y, size_average=False): the 11-tap SSIM and CS maps, differentiable w.r.t. x and y through the generic
+    backward with per-position upstream gradients."""
+
+    @staticmethod
+    def forward(ctx, win, data_range, use_padding, x, y):
+        maps = _ssim_map(x, y, win, data_range, use_padding, True)
+        imgs, _ = _dev_imgs((x, y))
+        ctx.save_for_backward(*imgs)
+        ctx.cfg, ctx.args = (data_range, use_padding), [(t.shape, t.device) for t in (x, y)]
+        ctx.set_materialize_grads(False)
+        return maps
+
+    @staticmethod
+    def backward(ctx, g_ssim, g_cs):
+        from . import loss as ML
+        x, y = ctx.saved_tensors
+        if g_ssim is None and g_cs is None:
+            return (None,) * 5
+        data_range, use_padding = ctx.cfg
+        dev = x.device
+        if use_padding:
+            x, y = _pad_dev(x, 5), _pad_dev(y, 5)
+        gm = [None if g is None else g.to(device=dev, dtype=torch.float32).reshape(x.shape[0], x.shape[1] - 10, x.shape[2] - 10)
+              for g in (g_ssim, g_cs)]
+        L.ensure_window_taps(11, 1.5)
+        dx, dy = ML._generic_bwd(x, y, data_range, 11, gm[0], gm[1], None, True, ctx.needs_input_grad[3],
+                                 ctx.needs_input_grad[4], sigma=1.5)
+        if use_padding:
+            dx = ML._pad_bwd_raw(dx, 5) if dx is not None else None
+            dy = ML._pad_bwd_raw(dy, 5) if dy is not None else None
+        return (None,) * 3 + tuple(None if d is None else d.view(s).to(dv) for d, (s, dv) in zip((dx, dy), ctx.args))
+
+
+class _MSSSIMFn(torch.autograd.Function):
+    """calc_msssim(x, y) of the pair (tr[slot], tr[2]) from the memo entry, differentiable w.r.t. x and y: per level the
+    SSIM backward of cs (levels 0..3) or ssim (level 4) with the chain-rule factor w_l * ms / v_l (0 where the level value
+    is below the 1e-7 clamp), then the pooling adjoints, as loss._MSSSIM.backward composes them.  The backward runs on the
+    generic kernels (double arithmetic), level values included: the product over five levels amplifies the error of
+    float32 level values and of the float32 strip kernels' CS gradient (on near-identical images a difference of nearly
+    equal terms) beyond the reference's own float32 error (2.3e-5 against 9.1e-6 of max|g| on ir_crop)."""
+
+    @staticmethod
+    def forward(ctx, tr, slot, win, data_range, use_padding, x, y):
+        out = _scalar(_rows(_msssim2(*tr, win, data_range, use_padding), x.device), slot)
+        imgs, _ = _dev_imgs(tr)
+        ctx.save_for_backward(imgs[slot], imgs[2])
+        ctx.cfg, ctx.args = (win, data_range, use_padding), [(t.shape, t.device) for t in (x, y)]
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        from . import loss as ML
+        lib = L.load()
+        x, y = ctx.saved_tensors
+        win, data_range, use_padding = ctx.cfg
+        want_x, want_y = ctx.needs_input_grad[5], ctx.needs_input_grad[6]
+        dev = x.device
+        xs, ys = [x], [y]
+        for _ in range(4):                      # the pyramid pools the unpadded level (metric.py:378-400)
+            xs.append(_halve_dev(xs[-1]))
+            ys.append(_halve_dev(ys[-1]))
+        levels = []
+        for xl, yl in zip(xs, ys):
+            k = min(int(win), *xl.shape[-2:])       # metric.py:323-325
+            p = k // 2 if use_padding else 0
+            levels.append((_pad_dev(xl, p), _pad_dev(yl, p), k, p) if p else (xl, yl, k, 0))
+        v = torch.stack([ML._generic_fwd(xl, yl, data_range, k, sigma=1.5)[:, 1 if lv < 4 else 0].mean()
+                         for lv, (xl, yl, k, _) in enumerate(levels)])
+        wts = torch.tensor(_MS_WEIGHTS, dtype=torch.float64, device=dev)
+        vc = v.clamp(min=1e-7)
+        ms = torch.prod(vc ** wts)
+        fac = (g.to(device=dev, dtype=torch.float64) * wts * ms / vc * (v >= 1e-7)).to(torch.float32)
+        grads = []
+        for lv, (xl, yl, k, p) in enumerate(levels):
+            gs, gc = (None, fac[lv]) if lv < 4 else (fac[lv], None)
+            d = _ssim_mean_grads(xl, yl, k, data_range, gs, gc, want_x, want_y, strip=False)
+            grads.append([ML._pad_bwd_raw(t, p) if (p and t is not None) else t for t in d])
+        out = []
+        for i in range(2):
+            if grads[0][i] is None:
+                out.append(None)
+                continue
+            for lv in range(4, 0, -1):
+                n, h, w = grads[lv - 1][i].shape
+                L.call(dev, lib.mmif_halve_bwd, grads[lv][i].data_ptr(), n, h, w, grads[lv - 1][i].data_ptr(), L.stream_int(dev))
+            shape, device = ctx.args[i]
+            out.append(grads[0][i].view(shape).to(device))
+        return (None,) * 5 + tuple(out)
+
+
 def _scalar(rows, idx, dtype=torch.float32):
     """0-dim tensor rows[0, idx] in the reference's dtype, on the device `rows` lives on (the caller's)."""
     return rows[0, idx].to(dtype)
@@ -451,8 +696,7 @@ def _single(t, what):
 
 def _stat1(img, idx_f, idx_a, idx_b):
     """A one-image statistic of `img`: column idx_f of the triple that has it as fused image, else of (img, img, img)."""
-    tr = _one(img)
-    return _scalar(_rows(_stats(*tr), img.device), idx_f)
+    return _stat(_one(img), idx_f, (2,), img)
 
 
 # 1. mean
@@ -483,7 +727,7 @@ def calc_sf(img):
 def calc_mse(img1, img2):
     _single(img1, 'calc_mse')
     tr, slot = _two(img1, img2)
-    return _scalar(_rows(_stats(*tr), img1.device), 4 + slot)
+    return _stat(tr, 4 + slot, (slot, 2), img1, img2)
 
 
 # 6. psnr — pure scalar arithmetic on the mse tensor, as in the reference (metric.py:72-76)
@@ -497,14 +741,14 @@ def calc_psnr(mse, L=1.0, root=False):
 def calc_cc(img1, img2):
     _single(img1, 'calc_cc')
     tr, slot = _two(img1, img2)
-    return _scalar(_rows(_stats(*tr), img1.device), 6 + slot)
+    return _stat(tr, 6 + slot, (slot, 2), img1, img2)
 
 
 # 8. scd
 def calc_scd(img1, img2, imgf):
     _single(img1, 'calc_scd')
     _triples.add(img1, img2, imgf)
-    return _scalar(_rows(_stats(img1, img2, imgf), img1.device), 8)
+    return _stat((img1, img2, imgf), 8, (0, 1, 2), img1, img2, imgf)
 
 
 # 9. en
@@ -553,8 +797,14 @@ def calc_Labf(img1, img2, imgf, L=1.5):
 def calc_ssim(img1, img2, win_size=11, data_range=255.0, use_padding=False, size_average=True, full=False):
     _single(img1, 'calc_ssim')
     if not size_average:
+        if _grad_wanted(img1, img2):
+            maps = _SSIMMapFn.apply(win_size, data_range, use_padding, img1, img2)
+            return maps if full else maps[0]
         return _ssim_map(img1, img2, win_size, data_range, use_padding, full)
     tr, slot = _two(img1, img2)
+    if _grad_wanted(img1, img2):
+        s, cs = _SSIMFn.apply(tr, slot, win_size, data_range, use_padding, img1, img2)
+        return (s, cs) if full else s
     r = _rows(_ssim2(*tr, win_size, data_range, use_padding), img1.device)
     if full:
         return _scalar(r, 2 * slot), _scalar(r, 2 * slot + 1)
@@ -586,6 +836,8 @@ def _ssim_map(img1, img2, win_size, data_range, use_padding, full):
 def calc_msssim(img1, img2, win_size=11, data_range=255.0, use_padding=False):
     _single(img1, 'calc_msssim')
     tr, slot = _two(img1, img2)
+    if _grad_wanted(img1, img2):
+        return _MSSSIMFn.apply(tr, slot, win_size, data_range, use_padding, img1, img2)
     return _scalar(_rows(_msssim2(*tr, win_size, data_range, use_padding), img1.device), slot)
 
 

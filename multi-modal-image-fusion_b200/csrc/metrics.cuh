@@ -39,6 +39,8 @@ enum {
 
 int launch_stats(const float* a, const float* b, const float* f, int N, int H, int W, double* out, long long ostride, MetricWs& ws,
                  cudaStream_t st);
+int launch_stats_bwd(const float* a, const float* b, const float* f, int N, int H, int W, const double* row, const float* gout,
+                     float* da, float* db, float* df, cudaStream_t st);
 int launch_hist(const float* a, const float* b, const float* f, int N, int H, int W, uint32_t* counts, double* ent,
                 long long estride, MetricWs& ws, cudaStream_t st);
 int launch_qabf(const float* a, const float* b, const float* f, int N, int H, int W, float L, double* out, long long ostride,

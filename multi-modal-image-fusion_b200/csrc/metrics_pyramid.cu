@@ -456,6 +456,17 @@ extern "C" int mmif_stats(const float* a, const float* b, const float* f, int N,
     return launch_stats(a, b, f, N, H, W, out, MMIF_ST_COUNT, w, (cudaStream_t)stream);
 }
 
+extern "C" int mmif_stats_bwd(const float* a, const float* b, const float* f, int N, int H, int W, const double* row,
+                              const float* gout, float* da, float* db, float* df, void* stream) {
+    int rc = check_imgs(a, b, f, N, H, W); if (rc) return rc;
+    if (!row || !gout) { set_error("null row or gout"); return MMIF_E_NULL; }
+    if ((((uintptr_t)row) & 7) || ((((uintptr_t)gout) | ((uintptr_t)da) | ((uintptr_t)db) | ((uintptr_t)df)) & 3)) {
+        set_error("row must be 8-byte, gout and the gradients 4-byte aligned");
+        return MMIF_E_ALIGN;
+    }
+    return launch_stats_bwd(a, b, f, N, H, W, row, gout, da, db, df, (cudaStream_t)stream);
+}
+
 extern "C" int mmif_hist(const float* a, const float* b, const float* f, int N, int H, int W, uint32_t* counts, double* ent,
                          void* ws, size_t ws_bytes, void* stream) {
     int rc = check_imgs(a, b, f, N, H, W); if (rc) return rc;

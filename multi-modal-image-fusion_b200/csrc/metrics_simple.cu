@@ -220,6 +220,187 @@ int launch_qabf(const float* a, const float* b, const float* f, int N, int H, in
     return launch_pixel_metrics(a, b, f, N, H, W, L, nullptr, 0, out, ostride, ws, st, q_raw);
 }
 
+// =============================================================================== statistics gradient
+// Gradient of sum_c gout[c] * stat[c] over the MMIF_ST_* columns of one batch row.  Every statistic except AG and SF is
+// a function of the batch means and (co)variances of (a, b, f), so its gradient w.r.t. an image x is affine in the
+// centred pixels: dx = c0[x] + K[x][a] (a - ma) + K[x][b] (b - mb) + K[x][f] (f - mf).  dC_xy / dx_i = (y_i - my) / P:
+// the mean terms cancel.  AG and SF add their forward-difference stencil terms to df.  Coefficients are formed once
+// per block in double; a zero sd or a 0/0 correlation makes its coefficients NaN, so NaN reaches every pixel, as the
+// reference's pow(0.5) at 0 and 0/0 correlations do under autograd.  A column whose gout is exactly 0 is skipped.
+struct StatsBwdCoef {
+    double c0[3], K[3][3], mu[3];
+    double kag, ksv, ksh;        // AG per-stencil factor, SF vertical / horizontal factors
+};
+
+// d/dx, d/dy of g * corr(x, y) (metric.py:80-91) with sx, sy the population sds and r the correlation.
+__device__ void cc_coef(StatsBwdCoef& c, int x, int y, double sx, double sy, double r, double g, double P) {
+    if (sx == 0.0 || sy == 0.0) {
+        const double nan = __longlong_as_double(0x7ff8000000000000ll);
+        c.K[x][x] += nan; c.K[x][y] += nan; c.K[y][x] += nan; c.K[y][y] += nan;
+        return;
+    }
+    const double m = g / (P * sx * sy);
+    c.K[x][y] += m; c.K[y][x] += m;
+    c.K[x][x] -= g * r / (P * sx * sx);
+    c.K[y][y] -= g * r / (P * sy * sy);
+}
+
+// d/d(src, other, f) of g * corr(f - src, other): one term of scd (metric.py:95-99).
+__device__ void scd_coef(StatsBwdCoef& c, int s, int o, double Css, double Coo, double Cff, double Csf, double Cof, double Cso,
+                         double g, double P) {
+    const double su = sqrt(fmax(Cff + Css - 2.0 * Csf, 0.0)), so = sqrt(Coo);
+    if (su == 0.0 || so == 0.0) {
+        const double nan = __longlong_as_double(0x7ff8000000000000ll);
+        for (int x = 0; x < 3; ++x) for (int y = 0; y < 3; ++y) c.K[x][y] += nan;
+        return;
+    }
+    const double r = (Cof - Cso) / (su * so);
+    const double A = g / (P * su * so), B = g * r / (P * su * su), C = g * r / (P * so * so);
+    // u = f - src, v = other:  gu = A (v - mv) - B (u - mu),  gv = A (u - mu) - C (v - mv);  df += gu, dsrc -= gu, dother += gv
+    c.K[2][o] += A; c.K[2][2] -= B; c.K[2][s] += B;
+    c.K[s][o] -= A; c.K[s][2] += B; c.K[s][s] -= B;
+    c.K[o][2] += A; c.K[o][s] -= A; c.K[o][o] -= C;
+}
+
+__device__ void stats_bwd_coef(StatsBwdCoef& c, const double* row, const float* gout, int N, int H, int W) {
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    const double P = (double)N * H * W;
+    const double ma = row[MMIF_ST_MEAN_A], mb = row[MMIF_ST_MEAN_B], mf = row[MMIF_ST_MEAN_F];
+    const double sa = row[MMIF_ST_SD_A], sb = row[MMIF_ST_SD_B], sf = row[MMIF_ST_SD];
+    // covariances from the correlations; a constant image has zero covariance with anything
+    const double Caf = (sa == 0.0 || sf == 0.0) ? 0.0 : row[MMIF_ST_CC_AF] * sa * sf;
+    const double Cbf = (sb == 0.0 || sf == 0.0) ? 0.0 : row[MMIF_ST_CC_BF] * sb * sf;
+    const double Cab = (sa == 0.0 || sb == 0.0) ? 0.0 : row[MMIF_ST_CC_AB] * sa * sb;
+    for (int x = 0; x < 3; ++x) { c.c0[x] = 0.0; for (int y = 0; y < 3; ++y) c.K[x][y] = 0.0; }
+    c.mu[0] = ma; c.mu[1] = mb; c.mu[2] = mf;
+    c.kag = c.ksv = c.ksh = 0.0;
+    double g[MMIF_ST_COUNT];
+    for (int i = 0; i < MMIF_ST_COUNT; ++i) g[i] = (double)gout[i];
+    if (g[MMIF_ST_MEAN_F] != 0.0) c.c0[2] += g[MMIF_ST_MEAN_F] / P;
+    if (g[MMIF_ST_SD] != 0.0) c.K[2][2] += (sf == 0.0) ? nan : g[MMIF_ST_SD] / (P * sf);
+    if (g[MMIF_ST_AG] != 0.0) c.kag = g[MMIF_ST_AG] / ((double)N * (H - 1) * (W - 1));
+    if (g[MMIF_ST_SF] != 0.0) {
+        const double v = row[MMIF_ST_SF];
+        c.ksv = (v == 0.0) ? nan : g[MMIF_ST_SF] / (v * ((double)N * (H - 1) * W));
+        c.ksh = (v == 0.0) ? nan : g[MMIF_ST_SF] / (v * ((double)N * H * (W - 1)));
+    }
+    for (int s = 0; s < 2; ++s) {                       // mse(src, f) = E[(src - f)^2] / 255^2 (metric.py:63-68)
+        const double gm = g[MMIF_ST_MSE_AF + s];
+        if (gm == 0.0) continue;
+        const double m = 2.0 * gm / (255.0 * 255.0 * P), d = m * (c.mu[s] - mf);
+        c.c0[s] += d; c.c0[2] -= d;
+        c.K[s][s] += m; c.K[s][2] -= m; c.K[2][s] -= m; c.K[2][2] += m;
+    }
+    if (g[MMIF_ST_CC_AF] != 0.0) cc_coef(c, 0, 2, sa, sf, row[MMIF_ST_CC_AF], g[MMIF_ST_CC_AF], P);
+    if (g[MMIF_ST_CC_BF] != 0.0) cc_coef(c, 1, 2, sb, sf, row[MMIF_ST_CC_BF], g[MMIF_ST_CC_BF], P);
+    if (g[MMIF_ST_CC_AB] != 0.0) cc_coef(c, 0, 1, sa, sb, row[MMIF_ST_CC_AB], g[MMIF_ST_CC_AB], P);
+    if (g[MMIF_ST_MEAN_A] != 0.0) c.c0[0] += g[MMIF_ST_MEAN_A] / P;
+    if (g[MMIF_ST_MEAN_B] != 0.0) c.c0[1] += g[MMIF_ST_MEAN_B] / P;
+    if (g[MMIF_ST_SD_A] != 0.0) c.K[0][0] += (sa == 0.0) ? nan : g[MMIF_ST_SD_A] / (P * sa);
+    if (g[MMIF_ST_SD_B] != 0.0) c.K[1][1] += (sb == 0.0) ? nan : g[MMIF_ST_SD_B] / (P * sb);
+    if (g[MMIF_ST_SCD] != 0.0) {                        // scd = cc(f - a, b) + cc(f - b, a)
+        scd_coef(c, 0, 1, sa * sa, sb * sb, sf * sf, Caf, Cbf, Cab, g[MMIF_ST_SCD], P);
+        scd_coef(c, 1, 0, sb * sb, sa * sa, sf * sf, Cbf, Caf, Cab, g[MMIF_ST_SCD], P);
+    }
+}
+
+// 0.5 / sqrt(0.5 (dx^2 + dy^2)) of one AG stencil (metric.py:44) in IEEE float32: a stencil with dx = dy = 0 gives inf,
+// so its dx * w and dy * w are 0 * inf = NaN on exactly its three pixels, as the reference's autograd gives.
+__device__ __forceinline__ float ag_w(float dx, float dy) {
+    const float q = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
+    return __fdiv_rn(0.5f, __fsqrt_rn(__fmul_rn(q, 0.5f)));
+}
+
+constexpr int kSbRows = 4;     // consecutive rows per thread: a 32 x 8 block covers a tile of 32 x 32 pixels
+constexpr int kSbBlocksPerSM = 3;
+
+// Gather form: the thread of pixel (i, j) writes its three outputs once, reading its own pixel, its neighbours and the
+// AG stencils (i, j), (i, j-1), (i-1, j) it belongs to.  No atomics: the result is deterministic.  A block forms the
+// coefficients once and then strides over the 32 x 32 tiles of the batch.
+__global__ void __launch_bounds__(256, kSbBlocksPerSM)
+stats_bwd_kernel(const float* __restrict__ A, const float* __restrict__ Bm, const float* __restrict__ F, int N, int H, int W,
+                 const double* __restrict__ row, const float* __restrict__ gout, float* da, float* db, float* df) {
+    __shared__ StatsBwdCoef cs;
+    if (threadIdx.x == 0 && threadIdx.y == 0) stats_bwd_coef(cs, row, gout, N, H, W);
+    __syncthreads();
+    const StatsBwdCoef& c = cs;
+    const bool stencil = df && (c.kag != 0.0 || c.ksv != 0.0 || c.ksh != 0.0);
+    const int tx = (W + 31) / 32, ty = (H + 8 * kSbRows - 1) / (8 * kSbRows);
+    const long long ntiles = (long long)tx * ty * N;
+    for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+        const int j = (int)(tile % tx) * 32 + threadIdx.x;
+        const int i0 = (int)((tile / tx) % ty) * (8 * kSbRows) + threadIdx.y * kSbRows;     // this thread's kSbRows rows
+        const size_t off = (size_t)(tile / ((long long)tx * ty)) * H * W;
+        if (j >= W || i0 >= H) continue;
+        const float *a = A + off, *b = Bm + off, *f = F + off;
+        // every load first (clamped addresses, unused values are ignored), so a thread has all of them in flight at once
+        const int jl = max(j - 1, 0), jr = min(j + 1, W - 1);
+        float va[kSbRows], vb[kSbRows], fc[kSbRows + 2], fl[kSbRows + 2], fr[kSbRows + 2];   // f rows i0-1 .. i0+kSbRows
+#pragma unroll
+        for (int k = 0; k < kSbRows; ++k) {
+            const size_t r = (size_t)min(i0 + k, H - 1) * W;
+            va[k] = __ldg(a + r + j); vb[k] = __ldg(b + r + j);
+        }
+#pragma unroll
+        for (int k = 0; k < kSbRows + 2; ++k) {
+            const size_t r = (size_t)min(max(i0 - 1 + k, 0), H - 1) * W;
+            fc[k] = __ldg(f + r + j);
+            fl[k] = stencil ? __ldg(f + r + jl) : 0.f;
+            fr[k] = stencil ? __ldg(f + r + jr) : 0.f;
+        }
+#pragma unroll
+        for (int k = 0; k < kSbRows; ++k) {
+            const int i = i0 + k;
+            if (i >= H) break;
+            const size_t q = off + (size_t)i * W + j;
+            const float fcc = fc[k + 1];
+            const double ca = (double)va[k] - c.mu[0], cb = (double)vb[k] - c.mu[1], cf = (double)fcc - c.mu[2];
+            if (da) da[q] = (float)(c.c0[0] + c.K[0][0] * ca + c.K[0][1] * cb + c.K[0][2] * cf);
+            if (db) db[q] = (float)(c.c0[1] + c.K[1][0] * ca + c.K[1][1] * cb + c.K[1][2] * cf);
+            if (!df) continue;
+            double v = c.c0[2] + c.K[2][0] * ca + c.K[2][1] * cb + c.K[2][2] * cf;
+            if (stencil) {
+                const bool up = i > 0, dn = i + 1 < H, lf = j > 0, rt = j + 1 < W;
+                const float fu = fc[k], fd = fc[k + 2], fle = fl[k + 1], fri = fr[k + 1];
+                if (c.ksv != 0.0 || c.ksh != 0.0) {          // sf (metric.py:50-59): dv = f(i+1,j) - f(i,j), dh = f(i,j+1) - f(i,j)
+                    const double dvu = up ? (double)fcc - fu : 0.0, dvd = dn ? (double)fd - fcc : 0.0;
+                    const double dhl = lf ? (double)fcc - fle : 0.0, dhr = rt ? (double)fri - fcc : 0.0;
+                    v += c.ksv * (dvu - dvd) + c.ksh * (dhl - dhr);
+                }
+                if (c.kag != 0.0) {                          // ag (metric.py:38-46) on the (H-1) x (W-1) stencil grid
+                    float t = 0.f;
+                    if (dn && rt) {                          // stencil (i, j): this pixel is its base
+                        const float dx = fri - fcc, dy = fd - fcc, w = ag_w(dx, dy);
+                        t = -(dx * w) - (dy * w);
+                    }
+                    if (dn && lf) {                          // stencil (i, j-1): this pixel is its right neighbour
+                        const float dx = fcc - fle, dy = fl[k + 2] - fle;
+                        t += dx * ag_w(dx, dy);
+                    }
+                    if (up && rt) {                          // stencil (i-1, j): this pixel is its lower neighbour
+                        const float dx = fr[k] - fu, dy = fcc - fu;
+                        t += dy * ag_w(dx, dy);
+                    }
+                    v += c.kag * (double)t;
+                }
+            }
+            df[q] = (float)v;
+        }
+    }
+}
+
+int launch_stats_bwd(const float* a, const float* b, const float* f, int N, int H, int W, const double* row, const float* gout,
+                     float* da, float* db, float* df, cudaStream_t st) {
+    if (H < 2 || W < 2) { set_error("stats_bwd: H and W must be >= 2"); return MMIF_E_SHAPE; }
+    if (!da && !db && !df) return MMIF_OK;
+    const long long tiles = (long long)ceil_div(W, 32) * ceil_div(H, 8 * kSbRows) * N;
+    const int grid = (int)(tiles < 148 * kSbBlocksPerSM ? tiles : 148 * kSbBlocksPerSM);
+    stats_bwd_kernel<<<grid, dim3(32, 8), 0, st>>>(a, b, f, N, H, W, row, gout, da, db, df);
+    mmif::count_launch(MMIF_CNT_METRIC);
+    MMIF_CUDA(cudaGetLastError());
+    return MMIF_OK;
+}
+
 // =============================================================================== histograms
 // Bin rule of torch.histc(im, 256, 0, 256) and np.histogram2d(.., 256, ((0,256),(0,256)))
 // (metric.py:113, 141-143): bin = floor(v) for 0 <= v < 256, v == 256 -> 255, -0.0 -> 0,
