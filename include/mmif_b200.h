@@ -279,6 +279,33 @@ int mmif_qabf(const float* a, const float* b, const float* f, int N, int H, int 
 int mmif_qabf_raw(const float* a, const float* b, const float* f, int N, int H, int W, float L,
                   double* out, void* ws, size_t ws_bytes, void* stream);
 
+/* Window-based fusion quality indices (definitions: oracle/quality_index.py): Piella & Heijmans' Q, Q_W, Q_E on every
+ * 8x8 box window and Yang et al.'s Q_Y on the 11x11 metric SSIM windows (sigma 1.5, data range 255).  One launch reads
+ * a, b, f once; the Sobel magnitudes of Q_E are formed on chip.  Per pair MMIF_QIDX_DOUBLES doubles: the four indices of
+ * the pair, then the raw sums behind them, so that a batch (one population) is a ratio of sums over all pairs:
+ *   Q = sum_term / box_windows;  Q_W = sum_cterm / sum_c (Q when sum_c == 0);
+ *   Q_E = Q_W * (sum_cterm_e / sum_c_e, or sum_term_e / box_windows when sum_c_e == 0);  Q_Y = sum_term_y / qy_windows.
+ * MMIF_E_NULL for a null image / out, MMIF_E_SHAPE unless N >= 1 and H, W >= 11, MMIF_E_ALIGN for an image pointer that
+ * is not 4-byte or an out / ws that is not 8-byte aligned, MMIF_E_WORKSPACE for a null or short ws (size from
+ * mmif_quality_index_workspace_bytes, which is 0 for a rejected shape; zero-filled once, left zeroed).
+ * No allocation, no synchronisation; one launch, counted under MMIF_CNT_METRIC. */
+enum {
+    MMIF_QIDX_Q = 0, MMIF_QIDX_QW = 1, MMIF_QIDX_QE = 2, MMIF_QIDX_QY = 3,
+    MMIF_QIDX_SUM_TERM = 4,       /* sum over box windows of lambda Q0(a,f) + (1 - lambda) Q0(b,f) */
+    MMIF_QIDX_BOX_WINDOWS = 5,    /* (H-7)(W-7) */
+    MMIF_QIDX_SUM_CTERM = 6,      /* sum of C * term, C = max(var a, var b) */
+    MMIF_QIDX_SUM_C = 7,
+    MMIF_QIDX_SUM_TERM_E = 8,     /* the same three on the Sobel magnitudes */
+    MMIF_QIDX_SUM_CTERM_E = 9,
+    MMIF_QIDX_SUM_C_E = 10,
+    MMIF_QIDX_SUM_TERM_Y = 11,    /* sum over the SSIM windows of the Q_Y terms */
+    MMIF_QIDX_QY_WINDOWS = 12     /* (H-10)(W-10) */
+};
+#define MMIF_QIDX_DOUBLES 13
+size_t mmif_quality_index_workspace_bytes(int N, int H, int W);
+int mmif_quality_index(const float* a, const float* b, const float* f, int N, int H, int W, double* out,
+                       void* ws, size_t ws_bytes, void* stream);
+
 /* calc_ssim(x,f,win,data_range,use_padding,full=True) (metric.py:316-364) for the two pairs
  * (a,f) and (b,f) -> per pair 4 doubles: ssim_af, cs_af, ssim_bf, cs_bf (global means). */
 int mmif_ssim(const float* a, const float* b, const float* f, int N, int H, int W, int win_size,

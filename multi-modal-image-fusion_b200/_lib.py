@@ -19,7 +19,7 @@ SYMBOLS = [
     'mmif_reflect_pad_bwd', 'mmif_metric_workspace_bytes', 'mmif_stats', 'mmif_hist', 'mmif_qabf', 'mmif_qabf_raw', 'mmif_ssim',
     'mmif_msssim', 'mmif_viff', 'mmif_eval_suite', 'mmif_eval_suite_host', 'mmif_ssim_maps', 'mmif_widen_u8', 'mmif_widen_u8_unit',
     'mmif_eval_suite_u8', 'mmif_eval_suite_u8_host', 'mmif_norm_workspace_bytes', 'mmif_norm_loss', 'mmif_norm_loss_bwd', 'mmif_test_post',
-    'mmif_widen', 'mmif_narrow', 'mmif_stats_bwd',
+    'mmif_widen', 'mmif_narrow', 'mmif_stats_bwd', 'mmif_quality_index_workspace_bytes', 'mmif_quality_index',
 ]
 
 COMBINE = {'max': 0, 'avg': 1}
@@ -27,6 +27,7 @@ NORM = {'l1': 1, 'l2': 2}
 LOSS_HEAD, LOSS_PER_SAMPLE = 4, 6
 ST_COUNT, EN_COUNT, HIST_WORDS = 16, 12, 3 * 256 + 2 * 65536
 MSSSIM_DOUBLES, VIFF_DOUBLES, EVAL_METRICS = 22, 26, 16
+QIDX_DOUBLES = 13
 HALF_DTYPES = {torch.bfloat16: 1, torch.float16: 2}       # MMIF_DTYPE_BF16, MMIF_DTYPE_F16
 
 
@@ -108,6 +109,9 @@ def load():
     lib.mmif_norm_loss_bwd.argtypes = [vp, sz, ci, cf, vp, vp, vp]
     lib.mmif_widen.argtypes = [vp, ci, sz, vp, vp]
     lib.mmif_narrow.argtypes = [vp, vp, sz, ci, vp, vp]
+    lib.mmif_quality_index_workspace_bytes.restype = sz
+    lib.mmif_quality_index_workspace_bytes.argtypes = [ci, ci, ci]
+    lib.mmif_quality_index.argtypes = [vp, vp, vp, ci, ci, ci, vp, vp, sz, vp]
     for name in SYMBOLS:
         getattr(lib, name)  # every declared symbol must be exported
     _lib = lib

@@ -18,6 +18,10 @@ w.r.t. every image argument.  A batch is one population, as for the values.  The
 itself (same memo entry, same launches, equal values); the gradient reaches exactly the tensors passed to the call,
 on their device (CPU inputs get CPU float32 gradients).  Qabf / Nabf / Labf, VIFF and the histogram family stay
 detached; the batched entries below take no gradient.
+
+Beside the reference's surface: ``calc_Q / calc_Qw / calc_Qe / calc_Qy``, the window-based quality indices of Piella &
+Heijmans and of Yang et al. (one ``mmif_quality_index`` launch per (a, b, f) triple, detached).  They are not in
+``__all__`` or ``eval_metrics``, so ``eval.py``'s ``import *`` and its spreadsheet are unchanged.
 """
 import ctypes
 import math
@@ -220,6 +224,14 @@ def _combine_batch(kind, val, part, extra):
         out[0, 1] = sc[:, 0].sum() / sc[:, 1].sum() + sc[:, 2].sum() / sc[:, 3].sum()
         out[0, 2:] = sc.reshape(-1)
         return out
+    if kind == 'qidx':                                                    # rows = mmif_quality_index: ratios of batch-wide sums
+        t = rows.sum(dim=0)
+        q = t[4] / t[5]
+        qw = q if t[7] == 0 else t[6] / t[7]
+        qw_e = t[8] / t[5] if t[10] == 0 else t[9] / t[10]
+        out = t.clone().view(1, -1)
+        out[0, 0], out[0, 1], out[0, 2], out[0, 3] = q, qw, qw * qw_e, t[11] / t[12]
+        return out
     raise L.MmifError(f'no batch rule for {kind}')
 
 
@@ -363,6 +375,23 @@ def _qabf(a, b, f, Lexp):
         return _call('mmif_qabf_raw', imgs, shape, 9, ctypes.c_float(Lexp))
     _triples.add(a, b, f)
     return _memo.get('qabf', (a, b, f), float(Lexp), run)
+
+
+def _qidx(a, b, f):
+    """memo entry of mmif_quality_index: per pair [Q, Q_W, Q_E, Q_Y, raw sums] (include/mmif_b200.h MMIF_QIDX_*)."""
+    def run():
+        lib = L.load()
+        imgs, (n, h, w), _ = _prep(a, b, f)
+        dev = imgs[0].device
+        nbytes = lib.mmif_quality_index_workspace_bytes(n, h, w)
+        if nbytes == 0:
+            raise L.MmifError(f'unsupported shape {(n, h, w)}: H and W must be >= 11')
+        out = torch.empty(n * L.QIDX_DOUBLES, dtype=torch.float64, device=dev)
+        ws = L.workspace(dev, nbytes, 'qidx', (n, h, w))
+        L.call(dev, lib.mmif_quality_index, imgs[0].data_ptr(), imgs[1].data_ptr(), imgs[2].data_ptr(), n, h, w,
+               out.data_ptr(), ws.data_ptr(), ws.numel(), L.stream_int(dev))
+        return out.view(n, L.QIDX_DOUBLES)
+    return _memo.get('qidx', (a, b, f), None, run)
 
 
 def _one(f):
@@ -791,6 +820,32 @@ def calc_Nabf(img1, img2, imgf, L=1.5, modified=True):
 def calc_Labf(img1, img2, imgf, L=1.5):
     _single(img1, 'calc_Labf')
     return _scalar(_rows(_qabf(img1, img2, imgf, L), img1.device), 2)
+
+
+# Window-based quality indices beside the reference's surface (definitions: oracle/quality_index.py).  The four share
+# one mmif_quality_index launch per (a, b, f) triple; detached, float32 0-dim results like calc_Qabf.
+def calc_Q(img1, img2, imgf):
+    """Piella & Heijmans' fusion quality index Q: the saliency-weighted Wang-Bovik index over every 8x8 window."""
+    _single(img1, 'calc_Q')
+    return _scalar(_rows(_qidx(img1, img2, imgf), img1.device), 0)
+
+
+def calc_Qw(img1, img2, imgf):
+    """Piella & Heijmans' weighted fusion quality index Q_W: windows weighted by max(var a, var b)."""
+    _single(img1, 'calc_Qw')
+    return _scalar(_rows(_qidx(img1, img2, imgf), img1.device), 1)
+
+
+def calc_Qe(img1, img2, imgf):
+    """Piella & Heijmans' edge-dependent fusion quality index Q_E = Q_W(images) * Q_W(Sobel magnitudes)."""
+    _single(img1, 'calc_Qe')
+    return _scalar(_rows(_qidx(img1, img2, imgf), img1.device), 2)
+
+
+def calc_Qy(img1, img2, imgf):
+    """Yang et al.'s SSIM-based fusion quality index Q_Y on the 11x11 metric SSIM windows."""
+    _single(img1, 'calc_Qy')
+    return _scalar(_rows(_qidx(img1, img2, imgf), img1.device), 3)
 
 
 # 16. ssim
